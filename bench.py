@@ -5,6 +5,8 @@
   python bench.py --impl reference --gpus N --steps K ...   reference arm: the CPU restatement of salva's own
                                                             algorithm (oracle/, kind "port": the Rust reference
                                                             cannot be built here) on the box's host cores
+  python bench.py --gpus 1 --steps K --dump-outputs DIR     also writes the fluid state after the last timed step as .npy
+                                                            files, so that two builds can be compared on identical inputs
 
 One "step" = one LiquidWorld::step (liquid_world.rs:62) of the whole world.
 Workload: N = 1 -> BASELINE.json configs[2], C3 (216^3 = 10 077 696 particles, DFSPH + Akinci2013 surface tension:
@@ -43,10 +45,9 @@ PER_GPU_NX = 64  # C4 slices: 64 x 250 x 250 = 4M particles per GPU
 
 
 def peaks():
-    p = os.path.join(ROOT, "MEASURED_PEAKS.json")
-    if os.path.exists(p):
-        return float(json.load(open(p))["hbm_gbs"]), "measured (MEASURED_PEAKS.json)"
-    return 6650.0, "fallback (B200_PROFILING.md)"
+    # Roofline denominator: median of 50 device-to-device copies of 4 GiB (bytes read + written), timed with CUDA events on an
+    # NVIDIA B200 at its 1000 W power limit (SM clock max 1965 MHz).  Kept here so every run divides by the same measured number.
+    return 6531.0, "measured: 4 GiB device-to-device copy, read + write, median of 50, NVIDIA B200 at 1000 W"
 
 
 class ClockSampler:
@@ -404,6 +405,25 @@ def timed_steps(world, sc, steps, barrier):
 
 timed_steps.per_step = []   # (step_ms, grid_ms) of every timed step on this rank: a one-off stall shows up here, not in the mean
 
+DUMP_MAX_PARTICLES = 1 << 21   # positions + velocities in f32: 48 MB, within the 64 MB that --dump-outputs may write
+
+
+def dump_outputs(world, fh, out_dir):
+    """What a caller of LiquidWorld::step receives after the last timed step: positions and velocities of every fluid in original
+    particle order, as out_dir/fluid<k>_{positions,velocities}.npy (f32).  Above DUMP_MAX_PARTICLES in all, fluid k keeps a fixed
+    sample (sorted indices drawn with seed k) of its share of that budget, so that two builds given the same arguments write the
+    same particles and can be compared array for array."""
+    counts = [world.num_particles(f) for f in fh]
+    total = sum(counts)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, (f, n) in enumerate(zip(fh, counts)):
+        p, v = world.read_fluid(f)
+        if total > DUMP_MAX_PARTICLES:
+            keep = np.sort(np.random.default_rng(k).choice(n, DUMP_MAX_PARTICLES * n // total, replace=False))
+            p, v = p[keep], v[keep]
+        np.save(os.path.join(out_dir, "fluid%d_positions.npy" % k), p)
+        np.save(os.path.join(out_dir, "fluid%d_velocities.npy" % k), v)
+
 
 def pick_grid_order(args, cfg, world_size):
     """Engine option Consts::xysub (SALVA_B200_XYSUB): 'rows' sorts the particles into (h/2 x h/2) columns with z running fastest, so
@@ -533,6 +553,8 @@ def native_arm(args, rank, world_size):
     clocks = sampler.stop()
     dev_s, wall = allmax([acc["step_ms"] * 1e-3, wall])
     value = nf * args.steps / dev_s
+    if args.dump_outputs:
+        dump_outputs(world, fh, args.dump_outputs)   # before the e2e loop below steps the same world again
 
     # ---- e2e: the reference-facing call sequence with HOST buffers, copies inside the timed region ----------------
     f0 = fh[0]
@@ -682,9 +704,16 @@ def main():
                     help="particle order of the counting sort: h = cells of width h (z fastest), rows = x / y binned at h / 2 (SALVA_B200_XYSUB=2); "
                          "auto (one GPU, DFSPH dam-break configs) = run both as short parity-checked probes and keep the faster one")
     ap.add_argument("--probe", action="store_true", help="internal: short run of one grid order (no CPU arm, no e2e loop)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write each fluid's positions and velocities as DIR/fluid<k>_{positions,velocities}.npy "
+                         "(f32, a fixed seeded sample above %d particles in all); one GPU, native arm only" % DUMP_MAX_PARTICLES)
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     world_size = int(os.environ.get("WORLD_SIZE", 1))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or world_size > 1):
+        ap.error("--dump-outputs needs the native arm on one GPU")
     if args.impl == "reference":
         reference_arm(args, rank, world_size)
         return 0

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -37,6 +38,46 @@ def test_native_arm_fails_loudly_without_a_gpu():
     r = _run("--steps", "1", "--warmup", "0", "--no-cpu", "--n", "8")
     assert r.returncode != 0
     assert not [ln for ln in r.stdout.splitlines() if ln.startswith("{") and '"value"' in ln]
+
+
+class _FakeWorld:
+    """num_particles / read_fluid of LiquidWorld over host arrays: particle i of fluid k sits at (k, i, -i)."""
+
+    def __init__(self, counts):
+        self.data = [np.stack([np.full(n, k), np.arange(n), -np.arange(n)], axis=1).astype(np.float32) for k, n in enumerate(counts)]
+
+    def num_particles(self, f):
+        return len(self.data[f])
+
+    def read_fluid(self, f):
+        return self.data[f].copy(), 2 * self.data[f]
+
+
+@pytest.mark.parametrize("counts", [(1000,), (3_000_000, 1_500_000)], ids=["whole", "sampled"])
+def test_dump_outputs_is_a_fixed_f32_sample_within_64_mb(tmp_path, counts):
+    sys.path.insert(0, ROOT)
+    import bench
+    for d in ("a", "b"):
+        bench.dump_outputs(_FakeWorld(counts), list(range(len(counts))), str(tmp_path / d))
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted("fluid%d_%s.npy" % (k, q) for k in range(len(counts)) for q in ("positions", "velocities"))
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= 64 << 20
+    for k, n in enumerate(counts):
+        p = np.load(tmp_path / "a" / ("fluid%d_positions.npy" % k))
+        v = np.load(tmp_path / "a" / ("fluid%d_velocities.npy" % k))
+        assert p.dtype == v.dtype == np.float32 and p.shape == v.shape and p.shape[1] == 3
+        assert (p[:, 0] == k).all() and np.array_equal(v, 2 * p)                 # rows stay whole, velocities match positions
+        idx = p[:, 1].astype(np.int64)
+        assert (np.diff(idx) > 0).all() and idx[-1] < n                          # distinct particles in original order
+        assert len(idx) == (n if sum(counts) <= bench.DUMP_MAX_PARTICLES else bench.DUMP_MAX_PARTICLES * n // sum(counts))
+        assert np.array_equal(p, np.load(tmp_path / "b" / ("fluid%d_positions.npy" % k)))   # same sample on every run
+
+
+def test_dump_outputs_is_refused_where_it_cannot_apply():
+    r = _run("--impl", "reference", "--steps", "1", "--dump-outputs", "unused")
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr
+    r = _run("--steps", "0")
+    assert r.returncode == 2 and "--steps" in r.stderr
 
 
 class _Args:
