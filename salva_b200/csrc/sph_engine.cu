@@ -27,10 +27,6 @@
 
 using namespace sphk;
 
-#ifndef SALVA_B200_TEX_DEFAULT
-#define SALVA_B200_TEX_DEFAULT true
-#endif
-
 namespace {
 
 // All worlds of a process share the module's __constant__ block; API calls are serialised per process
@@ -111,8 +107,7 @@ struct SlabArray {
     void* p;
     size_t elem;
 };
-sph_status slab_refresh_n(sph_world* w, const SlabArray* arrays, int n_arrays, cudaStream_t st = nullptr);
-sph_status slab_wait(sph_world* w);
+sph_status slab_refresh_n(sph_world* w, const SlabArray* arrays, int n_arrays);
 sph_status p2p_setup(sph_world* w);
 sph_status post_density_refresh(sph_world* w);
 sph_status slab_allreduce(sph_world* w, float* buf, size_t n);
@@ -152,10 +147,6 @@ struct SlabState {
     DBuf<unsigned long long> d_cnt64;
     DBuf<float4> out_l[3], out_r[3], col_l[3], col_r[3];
     bool global_valid = false;
-    // exchange / compute overlap: boundary columns first, their exchange on comm_st behind the interior launch
-    bool overlap = false, pending = false;  // measured (2xB200): 1.687 ms with overlap vs 1.660 without — the step is host-launch bound there
-    cudaStream_t comm_st = nullptr;
-    cudaEvent_t ev_ready = nullptr, ev_done = nullptr;
     // slot ranges of the current step (after the sort)
     uint32_t gl_count = 0, sl_begin = 0, sl_count = 0, sr_begin = 0, sr_count = 0, gr_begin = 0, gr_count = 0;
     uint32_t exp_ghost_l = 0, exp_ghost_r = 0, exp_send_l = 0, exp_send_r = 0;
@@ -180,7 +171,6 @@ struct sph_world {
     std::vector<BoundaryRec> bounds;
     size_t N = 0, B = 0;   // N = fluid particles OWNED by this world
     size_t Ntot = 0;       // slots of the sorted arrays during a step: owned + ghost (== N on one GPU)
-    bool single_launch = true;
     int protect_buf = -1;    // double-buffer index ensure_fluid_buffers() must not reallocate (it is being read)
     uint32_t own_begin = 0;  // first owned slot (ghost columns of a slab world sit at both ends of the sorted arrays)
     SlabState slab;
@@ -214,25 +204,18 @@ struct sph_world {
     DBuf<float> dens, alpha, kappa, divv, pred, bvol, bforce;
     DBuf<uint32_t> cid, rank, perm, cstart, bcid, brank, bperm, bstart, scan_aux[3], scan_aux_k[3];
     DBuf<uint32_t> nbr_f, nbr_b, cnt_f, cnt_b;
-    DBuf<float4> g_f;  // cached gradient scalars, one float4 per group of 4 contacts (same layout as nbr_f)
     // gather_backend 1 (sph_tile.cuh): 16-bit tile-local fluid contact indices
     DBuf<uint16_t> nbr16;
     uint32_t tile_slots = 2048;  // widest tile halo seen by the last neighbour build (local index space size)
     uint32_t n_tiles = 0;
     bool tile = false;
     // gather_backend 0: the second per-contact gather (v* / kappa) can go through the texture pipe
-    // uniform-mass packed gather records (sph_passes.cuh): pvx4 = (x,y,z,v*x), vyz2 = (v*y,v*z), pk4 = (x,y,z,kappa)
+    // uniform-mass packed gather records (sph_passes.cuh): pvx4 = (x,y,z,v*x), vyz2 = (v*y,v*z), pk4 = (x,y,z,kappa); their
+    // gathers are split evenly over the texture and LSU pipes (even / odd contacts)
     bool unimass = false;
-    int uni_eval_mode = 1, uni_upd_mode = 1;  // 1: gathers split evenly over the texture and LSU pipes (even / odd contacts), 2: the
-                                              // position record through the LSU pipe only (second record, if any, through TEX)
     DBuf<float4> pvx4, pk4;
     DBuf<float2> vyz2;
-    DBuf<Rec8> rec8, nrec8;  // 256-bit gather records: (pos, v*, rho) of the evaluations, (pos, normal, rho) of the Akinci force pass
-    int use_rec8 = 0;        // 0: off, 1: pressure-loop evaluations, 2: every evaluation of the step (+ fused XSPH / Akinci normals)
-    bool nrec_valid = false;
-    bool fuse_fold = true;  // fold + gravity + integrate in one pass when the force phase has nothing to launch
-    bool nbr_tex = false;  // experiment: odd neighbour-search candidates through the texture pipe (SALVA_B200_NBR_TEX)
-    bool fuse_akinci = true, nr4_valid = false;  // Akinci normals ride with a divergence evaluation (k_vel_divergence_xsph_u<.., 2>)
+    bool nr4_valid = false;  // Akinci normals rode with a divergence evaluation (k_vel_divergence_xsph_u<2>)
     cudaTextureObject_t tex_pvx = 0, tex_vyz = 0, tex_pk = 0;
     const void* tex_pvx_ptr = nullptr;
     const void* tex_vyz_ptr = nullptr;
@@ -247,16 +230,10 @@ struct sph_world {
     DBuf<float> ct_w[2], ct_g[2];
     DBuf<uint32_t> d_ticket;      // last-block ticket of the in-kernel error reduction (kept at 0 between launches)
     bool errsum_ready = false;    // the last evaluation launch already reduced its partials into errsum
-    DBuf<LoopCtl> d_ctl;          // device-side Jacobi loop control (sph_kernels.cuh LoopCtl)
-    LoopCtl* h_ctl = nullptr;     // pinned host mirror
-    bool device_loops = false;  // measured slower at C2 (gated no-op launches cost more than the syncs they save)
-    int use_gcache = 0;
-    bool fuse_div = true, fused_first_div = false;  // first compute_divergences evaluation rides with the density pass
-    bool fuse_xsph = true;    // XSPH sums ride with the stand-alone divergence evaluations (k_vel_divergence_xsph_u)
-    bool xs_valid = false;    // ... and the last evaluation of this step produced them
+    bool fused_first_div = false;  // the first compute_divergences evaluation rode with the density pass
+    bool xs_valid = false;    // the last divergence evaluation of this step produced the XSPH sums (k_vel_divergence_xsph_u)
     DBuf<float4> xs;
     uint32_t fused_nblk = 0;
-    bool use_tex = false;
     cudaTextureObject_t tex_vs = 0, tex_kappa = 0;
     const void* tex_vs_ptr = nullptr;
     const void* tex_kappa_ptr = nullptr;
@@ -281,9 +258,6 @@ struct sph_world {
     int nb[7] = {0, 0, 0, 0, 0, 0, 0};
     DBuf<int> d_nb;
     int xysub = 1;              // row order (Consts::xysub, SALVA_B200_XYSUB): x / y bins per cell; one GPU, gather backend 0 only
-    int zsub = 1;               // z-bins per cell of the counting sort (Consts::zsub, SALVA_B200_ZSUB).  Measured: 2..4 bins cut
-                                // the candidates by 17-25 % but k_neighbors does not get faster (-1 %) and the finer z order
-                                // costs the gather passes 10 % of their coalescing (profiles/r2_exp_k_zbins.md) => 1
 
     bool grid_ready = false;    // cstart/bstart + sorted arrays describe the last step's cell grid (AABB queries)
     bool ever_stepped = false;
@@ -344,10 +318,6 @@ inline int boundary_slot(const sph_world* w, uint32_t handle) {
     if (var##_slot_ < 0) return w->fail(SPH_ERR_INVALID, "bad boundary handle %u", (unsigned)(handle)); \
     const uint32_t var = (uint32_t)var##_slot_;
 
-// 256-bit gather records for EVERY evaluation of the step (SALVA_B200_REC8=2): single-fluid uniform-mass DFSPH on one GPU
-inline bool rec8_full(const sph_world* w) { return w->use_rec8 >= 2 && w->unimass && !w->slab.active && !w->tile && !w->use_gcache; }
-inline bool rec8_predict(const sph_world* w) { return w->use_rec8 >= 1 && w->unimass && !w->slab.active && !w->tile; }
-
 enum { SP_DIV_EVAL = 0, SP_DIV_UPD, SP_PRED, SP_PUPD, SP_COUNT };
 sph_status span_begin(sph_world* w, int slot) {
     if (w->n_spans == w->spans.size()) {
@@ -383,8 +353,6 @@ void fill_static_consts(sph_world* w) {
     c.h = w->h;
     c.inv_h = 1.0f / w->h;
     c.h2 = w->h * w->h;
-    c.zsub = w->tile ? 1 : w->zsub;
-    c.zsub_f = (float)c.zsub;
     c.xysub = (w->tile || w->slab.active) ? 1 : w->xysub;  // slab worlds cut x into cell columns of width h: plain cells there
     c.xysub_f = (float)c.xysub;
     c.h_reach = std::nextafter(w->h * 1.00001f, INFINITY);
@@ -417,7 +385,6 @@ void fill_static_consts(sph_world* w) {
     c.stride = w->stride;
     c.cap_f = w->cap_f;
     c.cap_b = w->cap_b;
-    c.use_gcache = w->use_gcache;
 }
 
 // ---- exclusive scan over n u32 (in place) -------------------------------------------------------
@@ -530,7 +497,6 @@ sph_status ensure_fluid_buffers(sph_world* w) {
     CU(w->pvx4.ensure(N));
     CU(w->pk4.ensure(N));
     CU(w->vyz2.ensure(N));
-    if (w->use_rec8) CU(w->rec8.ensure(N));
     CU(w->acc.ensure(N));
     CU(w->dens.ensure(N + 8));
     CU(w->alpha.ensure(N + 8));
@@ -544,13 +510,10 @@ sph_status ensure_fluid_buffers(sph_world* w) {
     CU(w->cnt_b.ensure(N));
     w->stride = (uint32_t)((N + 31) / 32 * 32);
     if (w->tile) CU(w->nbr16.ensure((size_t)w->cap_f * w->stride));
-    else {
-        CU(w->nbr_f.ensure((size_t)w->cap_f * w->stride));
-        CU(w->g_f.ensure((size_t)(w->cap_f / 4) * w->stride));
-    }
+    else CU(w->nbr_f.ensure((size_t)w->cap_f * w->stride));
     CU(w->nbr_b.ensure((size_t)w->cap_b * w->stride));
     uint32_t nblk = cdiv(std::max<size_t>(N, 1), PASS_T);
-    CU(w->partial.ensure((size_t)(nblk + 3) * std::max<size_t>(1, w->fluids.size())));  // +3: a slab pass may run as three sub-range launches
+    CU(w->partial.ensure((size_t)nblk * std::max<size_t>(1, w->fluids.size())));
     CU(w->errsum.ensure(MAX_FLUIDS));
     return SPH_OK;
 }
@@ -603,14 +566,10 @@ sph_status stage_up(sph_world* w) {
     w->staged = false;
     w->lists_valid = false;
     w->slab.global_valid = false;
-    {
-        const char* t = getenv("SALVA_B200_UNIMASS");
-        bool allow = t ? atoi(t) != 0 : true;
-        // a slab world takes the fast path on every rank or on none: volumes default to uniform there, and an empty
-        // slab inherits the constant from its first immigrant only through the classic path -> keep it simple: require
-        // particles with uniform volumes on this rank, otherwise fall back (all ranks are built by the same host code).
-        w->unimass = allow && !w->tile && w->desc.solver == SPH_SOLVER_DFSPH && w->fluids.size() == 1 && w->fluids[0].uniform_mass > 0.f;
-    }
+    // a slab world takes the fast path on every rank or on none: volumes default to uniform there, and an empty
+    // slab inherits the constant from its first immigrant only through the classic path -> keep it simple: require
+    // particles with uniform volumes on this rank, otherwise fall back (all ranks are built by the same host code).
+    w->unimass = !w->tile && w->desc.solver == SPH_SOLVER_DFSPH && w->fluids.size() == 1 && w->fluids[0].uniform_mass > 0.f;
     return SPH_OK;
 }
 
@@ -740,16 +699,15 @@ sph_status phase_grid(sph_world* w) {
     for (int a = 0; a < 3; ++a) dims[a] = (long long)hb[3 + a] - hb[a] + 3;  // one padding cell each side
     double ncell_d = (double)dims[0] * (double)dims[1] * (double)dims[2];
     if (ncell_d > 1.0e9) return w->fail(SPH_ERR_OOM, "dense cell grid too large: %lld x %lld x %lld cells of width h", dims[0], dims[1], dims[2]);
-    const int zsub = w->tile ? 1 : w->zsub;  // z-bins per cell (sph_kernels.cuh Consts::zsub)
     const int xys = (w->tile || w->slab.active) ? 1 : w->xysub;  // x / y bins per cell (row order, Consts::xysub)
-    if (ncell_d * zsub * xys * xys > 2.0e9) return w->fail(SPH_ERR_OOM, "dense cell grid too large: %lld x %lld x %lld cells of width h", dims[0], dims[1], dims[2]);
-    size_t ncell = (size_t)dims[0] * dims[1] * dims[2] * zsub * xys * xys;
+    if (ncell_d * xys * xys > 2.0e9) return w->fail(SPH_ERR_OOM, "dense cell grid too large: %lld x %lld x %lld cells of width h", dims[0], dims[1], dims[2]);
+    size_t ncell = (size_t)dims[0] * dims[1] * dims[2] * xys * xys;
     w->hc.ox = (hb[0] - 1) * xys;
     w->hc.oy = (hb[1] - 1) * xys;
-    w->hc.oz = (hb[2] - 1) * zsub;
+    w->hc.oz = hb[2] - 1;
     w->hc.nx = (int)dims[0] * xys;
     w->hc.ny = (int)dims[1] * xys;
-    w->hc.nz = (int)dims[2] * zsub;
+    w->hc.nz = (int)dims[2];
     w->hc.ntx = (int)((dims[0] - 2 + TILE_X - 1) / TILE_X);
     w->hc.nty = (int)((dims[1] - 2 + TILE_Y - 1) / TILE_Y);
     w->hc.ntz = (int)((dims[2] - 2 + TILE_Z - 1) / TILE_Z);
@@ -787,8 +745,7 @@ sph_status phase_grid(sph_world* w) {
             g.n1 = 3;
         }
         // reorder + v* = vel + vc (the divergence solve works on vel + vc carried over from the previous step, Appendix A.3.2) in one pass
-        LAUNCH(k_gather_vstar, N, 256, (uint32_t)N, w->perm.p, g, w->vs.p, w->unimass ? w->pvx4.p : nullptr, w->unimass ? w->vyz2.p : nullptr,
-               rec8_full(w) ? w->rec8.p : nullptr);
+        LAUNCH(k_gather_vstar, N, 256, (uint32_t)N, w->perm.p, g, w->vs.p, w->unimass ? w->pvx4.p : nullptr, w->unimass ? w->vyz2.p : nullptr);
         w->cur = c ^ 1;
     }
     // boundaries: same sort — reused while neither the boundaries nor the cell mapping changed (static tanks)
@@ -934,16 +891,11 @@ sph_status phase_neighbors(sph_world* w, sph_status (*speculative)(sph_world*) =
                 LAUNCH((k_neighbors_xy<false>), N, 128, w->pos[c].p, w->vel[c].p, w->cstart.p, w->bpos[bc].p, w->bvel[bc].p, w->bstart.p, w->nbr_f.p, w->nbr_b.p,
                        w->cnt_f.p, w->cnt_b.p, maxcnt);
         } else if (multi) {
-            LAUNCH((k_neighbors<true, false>), N, 128, w->pos[c].p, w->vel[c].p, w->cstart.p, w->bpos[bc].p, w->bvel[bc].p, w->bstart.p, w->nbr_f.p, w->nbr_b.p,
-                   w->cnt_f.p, w->cnt_b.p, maxcnt, (cudaTextureObject_t)0);
-        } else if (w->nbr_tex && w->unimass) {
-            // candidates from pvx4 (same x, y, z as pos4, fixed address => one texture object for the world's lifetime), odd ones via TEX
-            TRY(ensure_tex(w, &w->tex_pvx, &w->tex_pvx_ptr, w->pvx4.p, w->pvx4.cap));
-            LAUNCH((k_neighbors<false, true>), N, 128, w->pvx4.p, w->vel[c].p, w->cstart.p, w->bpos[bc].p, w->bvel[bc].p, w->bstart.p, w->nbr_f.p, w->nbr_b.p,
-                   w->cnt_f.p, w->cnt_b.p, maxcnt, w->tex_pvx);
+            LAUNCH((k_neighbors<true>), N, 128, w->pos[c].p, w->vel[c].p, w->cstart.p, w->bpos[bc].p, w->bvel[bc].p, w->bstart.p, w->nbr_f.p, w->nbr_b.p,
+                   w->cnt_f.p, w->cnt_b.p, maxcnt);
         } else {
-            LAUNCH((k_neighbors<false, false>), N, 128, w->pos[c].p, w->vel[c].p, w->cstart.p, w->bpos[bc].p, w->bvel[bc].p, w->bstart.p, w->nbr_f.p, w->nbr_b.p,
-                   w->cnt_f.p, w->cnt_b.p, maxcnt, (cudaTextureObject_t)0);
+            LAUNCH((k_neighbors<false>), N, 128, w->pos[c].p, w->vel[c].p, w->cstart.p, w->bpos[bc].p, w->bvel[bc].p, w->bstart.p, w->nbr_f.p, w->nbr_b.p,
+                   w->cnt_f.p, w->cnt_b.p, maxcnt);
         }
         int* hs = reinterpret_cast<int*>(w->h_pinned + 32);  // pinned: the copy is truly asynchronous
         CU(cudaMemcpyAsync(hs, w->d_scal.p + 7, 4 * sizeof(int), cudaMemcpyDeviceToHost, w->st));
@@ -974,10 +926,7 @@ sph_status phase_neighbors(sph_world* w, sph_status (*speculative)(sph_world*) =
         }
         if (early) CU(cudaMemsetAsync(w->d_scal.p + 7, 0, sizeof(int), w->st));  // error flag of the discarded speculative pass
         if (w->tile) CU(w->nbr16.ensure((size_t)w->cap_f * w->stride));
-        else {
-            CU(w->nbr_f.ensure((size_t)w->cap_f * w->stride));
-            CU(w->g_f.ensure((size_t)(w->cap_f / 4) * w->stride));
-        }
+        else CU(w->nbr_f.ensure((size_t)w->cap_f * w->stride));
         CU(w->nbr_b.ensure((size_t)w->cap_b * w->stride));
         fill_static_consts(w);
         TRY(upload_consts(w));
@@ -1053,7 +1002,7 @@ sph_status refresh_vstar(sph_world* w) {
 }
 // ghost refresh of the evaluation's output (kappa) — only needed when an update follows
 sph_status refresh_kappa(sph_world* w) {
-    if (!w->slab.active || w->slab.overlap) return SPH_OK;  // overlap mode: the evaluation exchanged kappa speculatively
+    if (!w->slab.active) return SPH_OK;
     if (w->unimass) return slab_refresh(w, w->pk4.p, sizeof(float4));
     return slab_refresh(w, w->kappa.p, sizeof(float));
 }
@@ -1068,8 +1017,8 @@ sph_status launch_density_alpha(sph_world* w) {
         TDISPATCH1(k_tile_density_alpha, multi, 16, cap, w->pos[c].p, w->vel[c].p, w->bpos[bc].p, w->cstart.p, cap, L, w->dens.p, w->alpha.p,
                    w->d_scal.p + 7);
     } else {
-        Lists L{reinterpret_cast<const uint4*>(w->nbr_f.p), w->nbr_b.p, w->cnt_f.p, w->cnt_b.p, w->g_f.p};
-        DISPATCH1(k_density_alpha, multi, N, PASS_T, w->pos[c].p, w->vel[c].p, w->bpos[bc].p, L, w->g_f.p, w->dens.p, w->alpha.p, w->d_scal.p + 7);
+        Lists L{reinterpret_cast<const uint4*>(w->nbr_f.p), w->nbr_b.p, w->cnt_f.p, w->cnt_b.p};
+        DISPATCH1(k_density_alpha, multi, N, PASS_T, w->pos[c].p, w->vel[c].p, w->bpos[bc].p, L, w->dens.p, w->alpha.p, w->d_scal.p + 7);
     }
     return SPH_OK;  // the ghost refresh of rho follows in post_density_refresh(), once the list-capacity check has passed
 }
@@ -1095,15 +1044,10 @@ sph_status post_density_refresh(sph_world* w) {
         }                                                                                         \
     } while (0)
 
-#define BOOL3(kern, b0, b1, b2, n, ...)                                                   \
+#define BOOL2(kern, b0, b1, n, ...)                                                                \
     do {                                                                                           \
-        if (b0) {                                                                                  \
-            if (b1) { if (b2) LAUNCH_R((kern<true, true, true>), n, __VA_ARGS__); else LAUNCH_R((kern<true, true, false>), n, __VA_ARGS__); } \
-            else    { if (b2) LAUNCH_R((kern<true, false, true>), n, __VA_ARGS__); else LAUNCH_R((kern<true, false, false>), n, __VA_ARGS__); } \
-        } else {                                                                                   \
-            if (b1) { if (b2) LAUNCH_R((kern<false, true, true>), n, __VA_ARGS__); else LAUNCH_R((kern<false, true, false>), n, __VA_ARGS__); } \
-            else    { if (b2) LAUNCH_R((kern<false, false, true>), n, __VA_ARGS__); else LAUNCH_R((kern<false, false, false>), n, __VA_ARGS__); } \
-        }                                                                                          \
+        if (b0) { if (b1) LAUNCH_R((kern<true, true>), n, __VA_ARGS__); else LAUNCH_R((kern<true, false>), n, __VA_ARGS__); }     \
+        else    { if (b1) LAUNCH_R((kern<false, true>), n, __VA_ARGS__); else LAUNCH_R((kern<false, false>), n, __VA_ARGS__); }   \
     } while (0)
 #define BOOL4(kern, b0, b1, b2, b3, n, ...)                                               \
     do {                                                                                           \
@@ -1122,115 +1066,58 @@ sph_status post_density_refresh(sph_world* w) {
     } while (0)
 
 
-// ---- slot ranges of a launch and the producer/exchange overlap of a slab world ---------------------------------------
-// A pass that PRODUCES data its neighbours' ghosts need (kappa after an evaluation, v* after an update) is launched on
-// the two boundary columns first; their exchange then runs on the communication stream while the interior launch
-// proceeds on the main stream.  Every pass waits for the previous exchange before it reads ghost slots.
-sph_status slab_wait(sph_world* w) {
-    SlabState& S = w->slab;
-    if (S.pending) {
-        CU(cudaStreamWaitEvent(w->st, S.ev_done, 0));
-        S.pending = false;
-    }
-    return SPH_OK;
-}
-template <class Fn>  // fn(Range rg, uint32_t first_partial_block) -> sph_status
-sph_status run_parts(sph_world* w, const SlabArray* arrays, int n_arrays, uint32_t* nblk_total, Fn fn) {
-    SlabState& S = w->slab;
-    TRY(slab_wait(w));
-    uint32_t off = 0;
-    w->single_launch = !(S.active && S.overlap && n_arrays != 0);  // one launch covers the pass -> in-kernel final reduction
-    auto part = [&](uint32_t b, uint32_t cnt) -> sph_status {
-        if (!cnt) return SPH_OK;
-        TRY(fn(Range{b, cnt}, off));
-        off += cdiv(cnt, PASS_T);
-        return SPH_OK;
-    };
-    const uint32_t N = (uint32_t)w->N;
-    if (!S.active || !S.overlap || n_arrays == 0) {
-        TRY(part(w->own_begin, N));
-        if (S.active && n_arrays) TRY(slab_refresh_n(w, arrays, n_arrays));
-    } else {
-        TRY(part(S.sl_begin, S.sl_count));
-        TRY(part(S.sr_begin, S.sr_count));
-        CU(cudaEventRecord(S.ev_ready, w->st));
-        CU(cudaStreamWaitEvent(S.comm_st, S.ev_ready, 0));
-        TRY(slab_refresh_n(w, arrays, n_arrays, S.comm_st));
-        CU(cudaEventRecord(S.ev_done, S.comm_st));
-        S.pending = true;
-        const uint32_t ib = S.sl_begin + S.sl_count, ie = S.has_right ? S.sr_begin : w->own_begin + N;
-        TRY(part(ib, ie > ib ? ie - ib : 0));
-    }
-    if (nblk_total) *nblk_total = off;
-    return SPH_OK;
-}
-
 // DFSPH: densities + alphas + the first divergence evaluation in one sweep (k_density_alpha_div)
 sph_status launch_density_alpha_div(sph_world* w, uint32_t* nblk) {
     int c = w->cur, bc = w->bcur;
     const bool multi = w->fluids.size() > 1;
-    Lists L{reinterpret_cast<const uint4*>(w->nbr_f.p), w->nbr_b.p, w->cnt_f.p, w->cnt_b.p, w->g_f.p};
+    Lists L{reinterpret_cast<const uint4*>(w->nbr_f.p), w->nbr_b.p, w->cnt_f.p, w->cnt_b.p};
     if (w->unimass) {
         TRY(ensure_tex(w, &w->tex_vyz, &w->tex_vyz_ptr, w->vyz2.p, w->vyz2.cap));
         TRY(ensure_tex(w, &w->tex_pvx, &w->tex_pvx_ptr, w->pvx4.p, w->pvx4.cap));
     } else {
         TRY(ensure_tex(w, &w->tex_vs, &w->tex_vs_ptr, w->vs.p, w->vs.cap));
     }
-    const size_t nf = std::max<size_t>(1, w->fluids.size());
-    sph_status rs = run_parts(w, nullptr, 0, nblk, [&](Range rg, uint32_t blk) -> sph_status {
-        float* partial = w->partial.p + (size_t)blk * nf;
-        uint32_t* tk = w->single_launch ? w->d_ticket.p : nullptr;
-        if (rec8_full(w))
-            LAUNCH_R(k_density_alpha_div_r8, rg, w->rec8.p, w->bpos[bc].p, L, w->dens.p, w->alpha.p, w->divv.p, w->pk4.p, partial, w->d_scal.p + 7, tk,
-                     w->errsum.p);
-        else if (w->unimass)
-            LAUNCH_R((k_density_alpha_div<false, true>), rg, w->pvx4.p, w->tex_pvx, w->vs.p, (cudaTextureObject_t)0, w->vyz2.p, w->tex_vyz, w->vel[c].p, w->bpos[bc].p, L,
-                     w->g_f.p, w->dens.p, w->alpha.p, w->divv.p, w->kappa.p, w->pk4.p, partial, w->d_scal.p + 7, tk, w->errsum.p);
-        else if (multi)
-            LAUNCH_R((k_density_alpha_div<true, false>), rg, w->pos[c].p, (cudaTextureObject_t)0, w->vs.p, w->tex_vs, w->vyz2.p, (cudaTextureObject_t)0, w->vel[c].p, w->bpos[bc].p,
-                     L, w->g_f.p, w->dens.p, w->alpha.p, w->divv.p, w->kappa.p, w->pk4.p, partial, w->d_scal.p + 7, tk, w->errsum.p);
-        else
-            LAUNCH_R((k_density_alpha_div<false, false>), rg, w->pos[c].p, (cudaTextureObject_t)0, w->vs.p, w->tex_vs, w->vyz2.p, (cudaTextureObject_t)0, w->vel[c].p, w->bpos[bc].p,
-                     L, w->g_f.p, w->dens.p, w->alpha.p, w->divv.p, w->kappa.p, w->pk4.p, partial, w->d_scal.p + 7, tk, w->errsum.p);
-        return SPH_OK;
-    });
-    w->errsum_ready = w->single_launch;
-    return rs;
+    const Range rg{w->own_begin, (uint32_t)w->N};
+    float* partial = w->partial.p;
+    uint32_t* tk = w->d_ticket.p;  // one launch covers the pass -> in-kernel final reduction
+    if (w->unimass)
+        LAUNCH_R((k_density_alpha_div<false, true>), rg, w->pvx4.p, w->tex_pvx, w->vs.p, (cudaTextureObject_t)0, w->vyz2.p, w->tex_vyz, w->vel[c].p, w->bpos[bc].p, L,
+                 w->dens.p, w->alpha.p, w->divv.p, w->kappa.p, w->pk4.p, partial, w->d_scal.p + 7, tk, w->errsum.p);
+    else if (multi)
+        LAUNCH_R((k_density_alpha_div<true, false>), rg, w->pos[c].p, (cudaTextureObject_t)0, w->vs.p, w->tex_vs, w->vyz2.p, (cudaTextureObject_t)0, w->vel[c].p, w->bpos[bc].p,
+                 L, w->dens.p, w->alpha.p, w->divv.p, w->kappa.p, w->pk4.p, partial, w->d_scal.p + 7, tk, w->errsum.p);
+    else
+        LAUNCH_R((k_density_alpha_div<false, false>), rg, w->pos[c].p, (cudaTextureObject_t)0, w->vs.p, w->tex_vs, w->vyz2.p, (cudaTextureObject_t)0, w->vel[c].p, w->bpos[bc].p,
+                 L, w->dens.p, w->alpha.p, w->divv.p, w->kappa.p, w->pk4.p, partial, w->d_scal.p + 7, tk, w->errsum.p);
+    *nblk = cdiv(rg.count, PASS_T);
+    w->errsum_ready = true;
+    return SPH_OK;
 }
 
 // compute_divergences (predict = false) / compute_predicted_densities (predict = true); returns #partials.
-// In a slab world with overlap the kappa ghosts are exchanged speculatively (the evaluation may turn out to be the
-// loop's last one) behind the interior launch; otherwise refresh_kappa() does it only when an update follows.
+// In a slab world refresh_kappa() exchanges the kappa ghosts afterwards, only when an update follows.
 // The fluid term of the FIRST force of a single-fluid DFSPH world can ride with the divergence evaluations when it is an
 // XSPHViscosity without a boundary term (see k_vel_divergence_xsph_u).
 bool xsph_fusable(const sph_world* w) {
-    if (!w->fuse_xsph || w->desc.solver != SPH_SOLVER_DFSPH || w->tile || !w->unimass || w->use_gcache || w->slab.active) return false;
+    if (w->desc.solver != SPH_SOLVER_DFSPH || w->tile || !w->unimass || w->slab.active) return false;
     if (w->fluids.size() != 1 || w->fluids[0].forces.empty()) return false;
     const sph_force_desc& d = w->fluids[0].forces[0].d;
     return d.kind == SPH_FORCE_XSPH_VISCOSITY && d.p[0] != 0.f && (d.p[1] == 0.f || w->B == 0);
 }
-// ... and on the default records (k_vel_divergence_xsph_u<.., 2>, one extra 4-byte gather of rho_j): single uniform-mass fluid
+// ... and on the default records (k_vel_divergence_xsph_u<2>, one extra 4-byte gather of rho_j): single uniform-mass fluid
 bool akinci_fusable_u(const sph_world* w) {
-    if (!w->fuse_akinci || w->desc.solver != SPH_SOLVER_DFSPH || w->tile || !w->unimass || w->use_gcache || w->slab.active || rec8_full(w)) return false;
+    if (w->desc.solver != SPH_SOLVER_DFSPH || w->tile || !w->unimass || w->slab.active) return false;
     if (w->fluids.size() != 1) return false;
     for (const ForceRec& fr : w->fluids[0].forces)
         if (fr.d.kind == SPH_FORCE_AKINCI2013_TENSION) return true;
     return false;
 }
-// Akinci2013 normals (positions + densities only) can ride with any stand-alone divergence evaluation of the step when the
-// evaluations gather the 256-bit records (rho_j comes with them): k_vel_divergence_r8<false, 2>.
-bool akinci_fusable(const sph_world* w) {
-    if (!rec8_full(w) || w->fluids.size() != 1) return false;
-    int n_akinci = 0;
-    for (const ForceRec& fr : w->fluids[0].forces) n_akinci += fr.d.kind == SPH_FORCE_AKINCI2013_TENSION;
-    return n_akinci >= 1;
-}
 
-sph_status launch_vel_divergence(sph_world* w, bool predict, uint32_t* nblk, const int* gate = nullptr) {
+sph_status launch_vel_divergence(sph_world* w, bool predict, uint32_t* nblk) {
     int c = w->cur, bc = w->bcur;
     const bool multi = w->fluids.size() > 1;
-    const bool xsf = !predict && !gate && xsph_fusable(w);
-    const bool akf = !predict && !gate && !xsf && akinci_fusable_u(w);
+    const bool xsf = !predict && xsph_fusable(w);
+    const bool akf = !predict && !xsf && akinci_fusable_u(w);
     if (xsf) CU(w->xs.ensure(std::max(w->Ntot, w->N)));
     if (akf) CU(w->normals.ensure(std::max(w->Ntot, w->N)));
     if (w->tile) {
@@ -1242,76 +1129,42 @@ sph_status launch_vel_divergence(sph_world* w, bool predict, uint32_t* nblk, con
         w->errsum_ready = false;
         return SPH_OK;
     }
-    Lists L{reinterpret_cast<const uint4*>(w->nbr_f.p), w->nbr_b.p, w->cnt_f.p, w->cnt_b.p, w->g_f.p};
+    Lists L{reinterpret_cast<const uint4*>(w->nbr_f.p), w->nbr_b.p, w->cnt_f.p, w->cnt_b.p};
     if (w->unimass) {
         TRY(ensure_tex(w, &w->tex_pvx, &w->tex_pvx_ptr, w->pvx4.p, w->pvx4.cap));
         TRY(ensure_tex(w, &w->tex_vyz, &w->tex_vyz_ptr, w->vyz2.p, w->vyz2.cap));
-    } else if (w->use_tex) {
+    } else {
         TRY(ensure_tex(w, &w->tex_vs, &w->tex_vs_ptr, w->vs.p, w->vs.cap));
     }
     float* out = predict ? w->pred.p : w->divv.p;
-    const size_t nf = std::max<size_t>(1, w->fluids.size());
-    SlabArray a[1] = {{w->unimass ? (void*)w->pk4.p : (void*)w->kappa.p, w->unimass ? sizeof(float4) : sizeof(float)}};
-    const int n_arrays = (w->slab.active && w->slab.overlap) ? 1 : 0;
-    sph_status rs = run_parts(w, a, n_arrays, nblk, [&](Range rg, uint32_t blk) -> sph_status {
-        float* partial = w->partial.p + (size_t)blk * nf;
-        uint32_t* tk = (w->single_launch && !gate) ? w->d_ticket.p : nullptr;
-        if (w->unimass) {
-            const bool ptex = w->uni_eval_mode == 1;
-            if (predict && rec8_predict(w) && !gate) {
-                LAUNCH_R((k_vel_divergence_r8<true, 0>), rg, w->rec8.p, w->bpos[bc].p, w->bvel[bc].p, L, w->dens.p, w->alpha.p, out, w->pk4.p, partial, w->dt,
-                         w->d_scal.p + 7, tk, w->errsum.p, (float4*)nullptr, 0.f, (Rec8*)nullptr);
-            } else if (!predict && rec8_full(w) && !gate) {
-                const float cf = xsf ? w->fluids[0].forces[0].d.p[0] : 0.f;
-                const bool akn = !xsf && akinci_fusable(w);
-                if (akn) CU(w->nrec8.ensure(std::max(w->Ntot, w->N)));
-                if (xsf) {
-                    LAUNCH_R((k_vel_divergence_r8<false, 1>), rg, w->rec8.p, w->bpos[bc].p, w->bvel[bc].p, L, w->dens.p, w->alpha.p, out, w->pk4.p, partial,
-                             w->dt, w->d_scal.p + 7, tk, w->errsum.p, w->xs.p, cf, (Rec8*)nullptr);
-                    w->xs_valid = true;
-                } else if (akn) {
-                    LAUNCH_R((k_vel_divergence_r8<false, 2>), rg, w->rec8.p, w->bpos[bc].p, w->bvel[bc].p, L, w->dens.p, w->alpha.p, out, w->pk4.p, partial,
-                             w->dt, w->d_scal.p + 7, tk, w->errsum.p, (float4*)nullptr, 0.f, w->nrec8.p);
-                    w->nrec_valid = true;
-                } else {
-                    LAUNCH_R((k_vel_divergence_r8<false, 0>), rg, w->rec8.p, w->bpos[bc].p, w->bvel[bc].p, L, w->dens.p, w->alpha.p, out, w->pk4.p, partial,
-                             w->dt, w->d_scal.p + 7, tk, w->errsum.p, (float4*)nullptr, 0.f, (Rec8*)nullptr);
-                }
-            } else if (predict) {
-                if (ptex) LAUNCH_R((k_vel_divergence_u<true, true>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, w->bvel[bc].p, L,
-                                   w->dens.p, w->alpha.p, out, w->pk4.p, partial, w->dt, w->d_scal.p + 7, gate, tk, w->errsum.p);
-                else LAUNCH_R((k_vel_divergence_u<true, false>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, w->bvel[bc].p, L,
-                              w->dens.p, w->alpha.p, out, w->pk4.p, partial, w->dt, w->d_scal.p + 7, gate, tk, w->errsum.p);
-            } else if (xsf) {
-                const float cf = w->fluids[0].forces[0].d.p[0];
-                if (ptex) LAUNCH_R((k_vel_divergence_xsph_u<true, 1>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, L, w->dens.p,
-                                   w->alpha.p, out, w->pk4.p, partial, tk, w->errsum.p, w->xs.p, cf);
-                else LAUNCH_R((k_vel_divergence_xsph_u<false, 1>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, L, w->dens.p,
-                              w->alpha.p, out, w->pk4.p, partial, tk, w->errsum.p, w->xs.p, cf);
-                w->xs_valid = true;
-            } else if (akf) {  // Akinci normals ride along: nr4 = (n, rho) for k_akinci_force_u
-                if (ptex) LAUNCH_R((k_vel_divergence_xsph_u<true, 2>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, L, w->dens.p,
-                                   w->alpha.p, out, w->pk4.p, partial, tk, w->errsum.p, w->normals.p, 0.f);
-                else LAUNCH_R((k_vel_divergence_xsph_u<false, 2>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, L, w->dens.p,
-                              w->alpha.p, out, w->pk4.p, partial, tk, w->errsum.p, w->normals.p, 0.f);
-                w->nr4_valid = true;
-            } else {
-                if (ptex) LAUNCH_R((k_vel_divergence_u<false, true>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, w->bvel[bc].p, L,
-                                   w->dens.p, w->alpha.p, out, w->pk4.p, partial, w->dt, w->d_scal.p + 7, gate, tk, w->errsum.p);
-                else LAUNCH_R((k_vel_divergence_u<false, false>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, w->bvel[bc].p, L,
-                              w->dens.p, w->alpha.p, out, w->pk4.p, partial, w->dt, w->d_scal.p + 7, gate, tk, w->errsum.p);
-            }
-        } else {
-            BOOL3(k_vel_divergence, multi, predict, w->use_tex, rg, w->pos[c].p, w->vs.p, w->tex_vs, w->vel[c].p, w->bpos[bc].p, w->bvel[bc].p, L, w->dens.p,
-                  w->alpha.p, out, w->kappa.p, partial, w->dt, w->d_scal.p + 7, gate, tk, w->errsum.p);
-        }
-        return SPH_OK;
-    });
-    w->errsum_ready = w->single_launch && !gate;
-    return rs;
+    const Range rg{w->own_begin, (uint32_t)w->N};
+    float* partial = w->partial.p;
+    uint32_t* tk = w->d_ticket.p;  // one launch covers the pass -> in-kernel final reduction
+    if (!w->unimass) {
+        BOOL2(k_vel_divergence, multi, predict, rg, w->pos[c].p, w->vs.p, w->tex_vs, w->vel[c].p, w->bpos[bc].p, w->bvel[bc].p, L, w->dens.p,
+              w->alpha.p, out, w->kappa.p, partial, w->dt, w->d_scal.p + 7, tk, w->errsum.p);
+    } else if (predict) {
+        LAUNCH_R((k_vel_divergence_u<true>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, w->bvel[bc].p, L,
+                 w->dens.p, w->alpha.p, out, w->pk4.p, partial, w->dt, w->d_scal.p + 7, tk, w->errsum.p);
+    } else if (xsf) {
+        const float cf = w->fluids[0].forces[0].d.p[0];
+        LAUNCH_R((k_vel_divergence_xsph_u<1>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, L, w->dens.p,
+                 w->alpha.p, out, w->pk4.p, partial, tk, w->errsum.p, w->xs.p, cf);
+        w->xs_valid = true;
+    } else if (akf) {  // Akinci normals ride along: nr4 = (n, rho) for k_akinci_force_u
+        LAUNCH_R((k_vel_divergence_xsph_u<2>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, L, w->dens.p,
+                 w->alpha.p, out, w->pk4.p, partial, tk, w->errsum.p, w->normals.p, 0.f);
+        w->nr4_valid = true;
+    } else {
+        LAUNCH_R((k_vel_divergence_u<false>), rg, w->pvx4.p, w->tex_pvx, w->vyz2.p, w->tex_vyz, w->bpos[bc].p, w->bvel[bc].p, L,
+                 w->dens.p, w->alpha.p, out, w->pk4.p, partial, w->dt, w->d_scal.p + 7, tk, w->errsum.p);
+    }
+    *nblk = cdiv(rg.count, PASS_T);
+    w->errsum_ready = true;
+    return SPH_OK;
 }
 // compute_velocity_changes_for_divergence (pressure = false) / compute_velocity_changes (pressure = true)
-sph_status launch_vel_update(sph_world* w, bool pressure, const int* gate = nullptr) {
+sph_status launch_vel_update(sph_world* w, bool pressure) {
     int c = w->cur, bc = w->bcur;
     const bool multi = w->fluids.size() > 1, bf = any_bforce(w);
     if (w->tile) {
@@ -1325,34 +1178,18 @@ sph_status launch_vel_update(sph_world* w, bool pressure, const int* gate = null
                        w->vs.p, w->bforce.p, w->inv_dt);
         return SPH_OK;
     }
-    Lists L{reinterpret_cast<const uint4*>(w->nbr_f.p), w->nbr_b.p, w->cnt_f.p, w->cnt_b.p, w->g_f.p};
-    if (w->unimass) TRY(ensure_tex(w, &w->tex_pk, &w->tex_pk_ptr, w->pk4.p, w->pk4.cap));
-    // the following evaluation gathers v*_j of ghosts (vs itself too: the velocity fold reads vel = v* for ghosts)
-    SlabArray a[3] = {{w->pvx4.p, sizeof(float4)}, {w->vyz2.p, sizeof(float2)}, {w->vs.p, sizeof(float4)}};
-    SlabArray a1[1] = {{w->vs.p, sizeof(float4)}};
-    return run_parts(w, w->unimass ? a : a1, w->unimass ? 3 : 1, nullptr, [&](Range rg, uint32_t) -> sph_status {
-        if (w->unimass) {
-            const bool ptex = w->uni_upd_mode == 1;
-            Rec8* rec = (!gate && ((pressure && rec8_predict(w)) || rec8_full(w))) ? w->rec8.p : nullptr;
-            if (w->uni_upd_mode == 3 && !rec && !gate) {
-                if (bf) {
-                    if (pressure) LAUNCH_R((k_vel_update_alt<true, true>), rg, w->pk4.p, w->tex_pk, w->vel[c].p, w->bpos[bc].p, L, w->vc[c].p, w->vs.p, w->pvx4.p, w->vyz2.p, w->bforce.p, w->inv_dt);
-                    else LAUNCH_R((k_vel_update_alt<true, false>), rg, w->pk4.p, w->tex_pk, w->vel[c].p, w->bpos[bc].p, L, w->vc[c].p, w->vs.p, w->pvx4.p, w->vyz2.p, w->bforce.p, w->inv_dt);
-                } else {
-                    if (pressure) LAUNCH_R((k_vel_update_alt<false, true>), rg, w->pk4.p, w->tex_pk, w->vel[c].p, w->bpos[bc].p, L, w->vc[c].p, w->vs.p, w->pvx4.p, w->vyz2.p, w->bforce.p, w->inv_dt);
-                    else LAUNCH_R((k_vel_update_alt<false, false>), rg, w->pk4.p, w->tex_pk, w->vel[c].p, w->bpos[bc].p, L, w->vc[c].p, w->vs.p, w->pvx4.p, w->vyz2.p, w->bforce.p, w->inv_dt);
-                }
-                return SPH_OK;
-            }
-            BOOL3(k_vel_update_u, bf, pressure, ptex, rg, w->pk4.p, w->tex_pk, w->vel[c].p, w->bpos[bc].p, L, w->vc[c].p, w->vs.p, w->pvx4.p, w->vyz2.p,
-                  rec, w->dens.p, w->bforce.p, w->inv_dt, gate);
-        } else {
-            // measured (profiles/r1_v1_*): the texture pipe helps the float4 v* gather (-12 %) but not the 4-byte kappa gather
-            BOOL4(k_vel_update, multi, bf, pressure, false, rg, w->pos[c].p, w->vel[c].p, w->bpos[bc].p, L, w->kappa.p, w->tex_kappa, w->vc[c].p, w->vs.p,
-                  w->bforce.p, w->inv_dt, gate);
-        }
-        return SPH_OK;
-    });
+    Lists L{reinterpret_cast<const uint4*>(w->nbr_f.p), w->nbr_b.p, w->cnt_f.p, w->cnt_b.p};
+    const Range rg{w->own_begin, (uint32_t)w->N};
+    if (w->unimass) {
+        TRY(ensure_tex(w, &w->tex_pk, &w->tex_pk_ptr, w->pk4.p, w->pk4.cap));
+        BOOL2(k_vel_update_u, bf, pressure, rg, w->pk4.p, w->tex_pk, w->vel[c].p, w->bpos[bc].p, L, w->vc[c].p, w->vs.p, w->pvx4.p, w->vyz2.p,
+              w->bforce.p, w->inv_dt);
+    } else {
+        // measured (profiles/r1_v1_*): the texture pipe helps the float4 v* gather (-12 %) but not the 4-byte kappa gather
+        BOOL4(k_vel_update, multi, bf, pressure, false, rg, w->pos[c].p, w->vel[c].p, w->bpos[bc].p, L, w->kappa.p, w->tex_kappa, w->vc[c].p, w->vs.p,
+              w->bforce.p, w->inv_dt);
+    }
+    return refresh_vstar(w);  // the following evaluation gathers v*_j of ghosts
 }
 
 // ---- ParticlesContacts materialisation + the context-style host plugin call (nonpressure_force.rs:15-27) ---------------
@@ -1472,7 +1309,7 @@ sph_status phase_forces(sph_world* w) {
     size_t N = w->N;
     int c = w->cur, bc = w->bcur;
     const bool multi = w->fluids.size() > 1, bf = any_bforce(w);
-    Lists L{reinterpret_cast<const uint4*>(w->nbr_f.p), w->nbr_b.p, w->cnt_f.p, w->cnt_b.p, w->g_f.p};
+    Lists L{reinterpret_cast<const uint4*>(w->nbr_f.p), w->nbr_b.p, w->cnt_f.p, w->cnt_b.p};
     TileLists TL{w->nbr16.p, w->nbr_b.p, w->cnt_f.p, w->cnt_b.p};
     for (size_t f = 0; f < w->fluids.size(); ++f)
         for (ForceRec& fr : w->fluids[f].forces) {
@@ -1512,11 +1349,6 @@ sph_status phase_forces(sph_world* w) {
                                    (uint32_t)f);
                         TDISPATCH2(k_tile_akinci_force, multi, bf, sb2, cap2, w->pos[c].p, w->vel[c].p, w->bpos[bc].p, w->cstart.p, cap2, TL, w->dens.p,
                                    w->normals.p, w->acc.p, w->bforce.p, (uint32_t)f, p[0], p[1], coh_norm, h6_64, adh_norm);
-                        break;
-                    }
-                    if (w->nrec_valid && f == 0) {  // normals came with a divergence evaluation, in the one-gather record of the force pass
-                        if (bf) LAUNCH((k_akinci_force_r8<true>), N, PASS_T, w->nrec8.p, w->bpos[bc].p, L, w->acc.p, w->bforce.p, p[0], p[1], coh_norm, h6_64, adh_norm);
-                        else LAUNCH((k_akinci_force_r8<false>), N, PASS_T, w->nrec8.p, w->bpos[bc].p, L, w->acc.p, w->bforce.p, p[0], p[1], coh_norm, h6_64, adh_norm);
                         break;
                     }
                     if (w->nr4_valid && f == 0) {  // normals (and rho, in .w) came with a divergence evaluation
@@ -1594,65 +1426,6 @@ void timestep_advance(sph_world* w, float total) {
     w->inv_dt = total == 0.f ? 0.f : 1.0f / total;
 }
 
-// One Jacobi loop of DFSPHSolver (divergence_solve :466-503 when pressure == false, pressure_solve :432-464 otherwise)
-// with the break decision taken on the device: iterations are enqueued SPEC at a time, kernels past the break are
-// gated off, and the host synchronises once per batch to learn whether the loop has ended.
-sph_status jacobi_loop_device(sph_world* w, bool pressure, bool first_eval_done, uint32_t first_nblk, float tol, uint32_t min_iter, uint32_t max_iter,
-                              int forced, uint32_t* n_upd, uint32_t* n_eval, float* last_err) {
-    LoopCtl hc;
-    memset(&hc, 0, sizeof hc);
-    hc.active = 1;
-    hc.tol = tol;
-    hc.min_iter = min_iter;
-    hc.max_iter = forced >= 0 ? (uint32_t)forced + 1 : max_iter;
-    hc.forced = forced;
-    hc.n_fluids = (int)w->fluids.size();
-    for (int f = 0; f < hc.n_fluids; ++f) {
-        double n = w->slab.active ? (double)w->slab.global_n : (double)w->fluids[f].n;
-        hc.inv_count[f] = n > 0 ? (float)(1.0 / n) : 0.f;
-    }
-    if (hc.max_iter == 0) {
-        *n_upd = *n_eval = 0;
-        return SPH_OK;
-    }
-    *w->h_ctl = hc;
-    CU(cudaMemcpyAsync(w->d_ctl.p, w->h_ctl, sizeof(LoopCtl), cudaMemcpyHostToDevice, w->st));
-    const int* g_active = &w->d_ctl.p->active;
-    const int* g_update = &w->d_ctl.p->do_update;
-    const int nf = hc.n_fluids;
-    const uint32_t SPEC = 2;  // iterations enqueued per host sync (typical loops run 1-2 updates)
-    uint32_t enq = 0;
-    bool first = true;
-    for (;;) {
-        for (uint32_t s = 0; s < SPEC && enq < hc.max_iter; ++s, ++enq) {
-            uint32_t nblk = first_nblk;
-            if (!(first && first_eval_done)) {
-                TRY(span_begin(w, pressure ? SP_PRED : SP_DIV_EVAL));
-                TRY(launch_vel_divergence(w, pressure, &nblk, g_active));
-                TRY(span_end(w));
-            }
-            first = false;
-            k_reduce_partials<<<nf, 256, 0, w->st>>>(w->partial.p, nblk, nf, w->errsum.p);
-            w->launches++;
-            TRY(slab_allreduce(w, w->errsum.p, nf));
-            k_loop_decide<<<1, 32, 0, w->st>>>(w->d_ctl.p, w->errsum.p);
-            w->launches++;
-            TRY(refresh_kappa(w));
-            TRY(span_begin(w, pressure ? SP_PUPD : SP_DIV_UPD));
-            TRY(launch_vel_update(w, pressure, g_update));
-            TRY(span_end(w));
-        }
-        CU(cudaMemcpyAsync(w->h_ctl, w->d_ctl.p, sizeof(LoopCtl), cudaMemcpyDeviceToHost, w->st));
-        CU(cudaStreamSynchronize(w->st));
-        if (!w->h_ctl->active || enq >= hc.max_iter) break;
-    }
-    // `for i in 0..max`: when the loop ran out of iterations the last update is not followed by an evaluation
-    *n_upd = w->h_ctl->iter;
-    *n_eval = w->h_ctl->n_eval;
-    *last_err = w->h_ctl->last_err;
-    return SPH_OK;
-}
-
 // DFSPHSolver::step dfsph_solver.rs:667-708
 sph_status dfsph_step(sph_world* w, float dt_total, const float g[3]) {
     size_t N = w->N;
@@ -1663,15 +1436,8 @@ sph_status dfsph_step(sph_world* w, float dt_total, const float g[3]) {
     // divergence_solve :466-503 (uses the PREVIOUS step's inv_dt; 0 on the first step)
     w->stats.n_divergence_iter = w->stats.n_divergence_eval = 0;
     w->xs_valid = false;
-    w->nrec_valid = false;
     w->nr4_valid = false;
     uint32_t maxit = w->force_div >= 0 ? (uint32_t)w->force_div + 1 : w->desc.max_divergence_iter;
-    const bool dev_loops = w->device_loops && !w->tile;
-    if (dev_loops && w->force_div < 0) {
-        TRY(jacobi_loop_device(w, false, w->fused_first_div, w->fused_nblk, w->desc.max_divergence_error * w->inv_dt * 0.01f, w->desc.min_divergence_iter,
-                               w->desc.max_divergence_iter, -1, &w->stats.n_divergence_iter, &w->stats.n_divergence_eval, &w->stats.last_divergence_error));
-        maxit = 0;
-    }
     for (uint32_t i = 0; i < maxit; ++i) {
         if (i == 0 && w->fused_first_div) {
             nblk = w->fused_nblk;  // evaluation 0 was computed by k_density_alpha_div
@@ -1703,11 +1469,9 @@ sph_status dfsph_step(sph_world* w, float dt_total, const float g[3]) {
     }
     CU(cudaEventRecord(w->ev[EV_DIV], w->st));
     // update_velocities :422-430, zero vc :689-691, acc += gravity :574-578
-    TRY(slab_wait(w));
-    const bool r8 = rec8_predict(w);
     // nothing to launch in the force phase (no plugin at all, or only the XSPH whose sums rode with the divergence loop)?  Then
-    // fold, acceleration and integration are one streaming pass (SALVA_B200_FUSE_FOLD=0 keeps them apart)
-    bool quiet_forces = w->fuse_fold && !r8;
+    // fold, acceleration and integration are one streaming pass
+    bool quiet_forces = true;
     for (size_t f = 0; f < w->fluids.size() && quiet_forces; ++f)
         for (const ForceRec& fr : w->fluids[f].forces)
             if (!(w->xs_valid && f == 0 && &fr == &w->fluids[0].forces[0] && fr.d.kind == SPH_FORCE_XSPH_VISCOSITY)) quiet_forces = false;
@@ -1727,18 +1491,13 @@ sph_status dfsph_step(sph_world* w, float dt_total, const float g[3]) {
         CU(cudaEventRecord(w->ev[EV_FORCES], w->st));
         timestep_advance(w, dt_total);  // :702
         LAUNCH(k_integrate_acc, N, 256, w->vel[c].p, w->vc[c].p, w->vs.p, w->acc.p, w->dt, w->unimass ? w->pvx4.p : nullptr,
-               w->unimass ? w->vyz2.p : nullptr, w->pos[c].p, r8 ? w->rec8.p : nullptr, w->dens.p);
+               w->unimass ? w->vyz2.p : nullptr);
     }
     TRY(refresh_vstar(w));
     CU(cudaEventRecord(w->ev[EV_INTEG], w->st));
     // pressure_solve :432-464
     w->stats.n_pressure_iter = w->stats.n_pressure_eval = 0;
     maxit = w->force_press >= 0 ? (uint32_t)w->force_press + 1 : w->desc.max_pressure_iter;
-    if (dev_loops && w->force_press < 0) {
-        TRY(jacobi_loop_device(w, true, false, 0, w->desc.max_density_error, w->desc.min_pressure_iter, w->desc.max_pressure_iter, -1,
-                               &w->stats.n_pressure_iter, &w->stats.n_pressure_eval, &w->stats.last_density_error));
-        maxit = 0;
-    }
     for (uint32_t i = 0; i < maxit; ++i) {
         TRY(span_begin(w, SP_PRED));
         TRY(launch_vel_divergence(w, true, &nblk));
@@ -1761,7 +1520,6 @@ sph_status dfsph_step(sph_world* w, float dt_total, const float g[3]) {
         w->stats.n_pressure_iter++;
     }
     CU(cudaEventRecord(w->ev[EV_PRESS], w->st));
-    TRY(slab_wait(w));  // a speculative exchange may still be in flight: it must land before the arrays are reused
     {
         static const int init[7] = {INT_MAX, INT_MAX, INT_MAX, INT_MIN, INT_MIN, INT_MIN, 0};
         CU(w->d_nb.ensure(8));
@@ -1827,7 +1585,7 @@ sph_status world_step(sph_world* w, float dt, const float g[3], const sph_coupli
     TRY(phase_neighbors(w, [](sph_world* w) -> sph_status {
         w->fused_first_div = false;
         if (w->N) {
-            if (w->desc.solver == SPH_SOLVER_DFSPH && !w->tile && w->fuse_div) {
+            if (w->desc.solver == SPH_SOLVER_DFSPH && !w->tile) {
                 TRY(launch_density_alpha_div(w, &w->fused_nblk));
                 w->fused_first_div = true;
             } else {
@@ -1944,32 +1702,13 @@ sph_status sph_world_create(const sph_world_desc* desc, sph_world** out) {
     w->desc = *desc;
     w->h = desc->particle_radius * desc->smoothing_factor * 2.0f;  // liquid_world.rs:44
     w->tile = desc->gather_backend == 1 && desc->solver == SPH_SOLVER_DFSPH;  // the tile backend covers the DFSPH passes only
-    if (desc->kernel_density || desc->kernel_gradient) w->use_gcache = 0;
-    if (const char* t = getenv("SALVA_B200_DEVICE_LOOPS")) w->device_loops = atoi(t) != 0;
-#if SPH_GCACHE
-    if (const char* t = getenv("SALVA_B200_GCACHE")) w->use_gcache = atoi(t);
-#endif
-    if (const char* t = getenv("SALVA_B200_REC8")) w->use_rec8 = atoi(t);
-    if (const char* t = getenv("SALVA_B200_FUSE_DIV")) w->fuse_div = atoi(t) != 0;
-    if (const char* t = getenv("SALVA_B200_FUSE_XSPH")) w->fuse_xsph = atoi(t) != 0;
-    if (const char* t = getenv("SALVA_B200_FUSE_AKINCI")) w->fuse_akinci = atoi(t) != 0;
-    if (const char* t = getenv("SALVA_B200_NBR_TEX")) w->nbr_tex = atoi(t) != 0;
-    if (const char* t = getenv("SALVA_B200_FUSE_FOLD")) w->fuse_fold = atoi(t) != 0;
-    if (const char* t = getenv("SALVA_B200_ZSUB")) w->zsub = std::min(8, std::max(1, atoi(t)));
     if (const char* t = getenv("SALVA_B200_XYSUB")) w->xysub = std::min(4, std::max(1, atoi(t)));
-    if (const char* t = getenv("SALVA_B200_UNI_EVAL")) w->uni_eval_mode = atoi(t);
-    if (const char* t = getenv("SALVA_B200_UNI_UPD")) w->uni_upd_mode = atoi(t);
-    {
-        const char* t = getenv("SALVA_B200_TEX");
-        w->use_tex = t ? atoi(t) != 0 : SALVA_B200_TEX_DEFAULT;
-    }
     memset(&w->hc, 0, sizeof w->hc);
     memset(&w->stats, 0, sizeof w->stats);
     bool ok = cudaStreamCreateWithFlags(&w->st, cudaStreamNonBlocking) == cudaSuccess;
     for (int i = 0; ok && i < EV_COUNT; ++i) ok = cudaEventCreate(&w->ev[i]) == cudaSuccess;
     ok = ok && cudaEventCreateWithFlags(&w->ev_lists, cudaEventDisableTiming) == cudaSuccess;
     ok = ok && cudaMallocHost(&w->h_pinned, 64 * sizeof(float)) == cudaSuccess;
-    ok = ok && cudaMallocHost(&w->h_ctl, sizeof(LoopCtl)) == cudaSuccess && w->d_ctl.ensure(1) == cudaSuccess;
     ok = ok && w->d_scal.ensure(16) == cudaSuccess && w->d_cnt.ensure(2) == cudaSuccess;
     ok = ok && w->d_ticket.ensure(4) == cudaSuccess && cudaMemset(w->d_ticket.p, 0, 4 * sizeof(uint32_t)) == cudaSuccess;
     if (!ok) {
@@ -1996,7 +1735,7 @@ void sph_world_destroy(sph_world* w) {
     w->bstart.release();
     for (auto& a : w->scan_aux) a.release();
     for (auto& a : w->scan_aux_k) a.release();
-    w->nbr_f.release(); w->g_f.release(); w->nbr16.release(); w->nbr_b.release(); w->cnt_f.release(); w->cnt_b.release();
+    w->nbr_f.release(); w->nbr16.release(); w->nbr_b.release(); w->cnt_f.release(); w->cnt_b.release();
     w->partial.release(); w->errsum.release(); w->d_scal.release(); w->d_cnt.release();
     w->o_a.release(); w->o_b.release(); w->o_c.release(); w->o_mass.release(); w->o_fid.release();
     iisph_release(w);
@@ -2006,7 +1745,7 @@ void sph_world_destroy(sph_world* w) {
         for (auto& fr : f.forces) elasticity_release(fr);
     for (cudaTextureObject_t t : {w->tex_pvx, w->tex_vyz, w->tex_pk})
         if (t) cudaDestroyTextureObject(t);
-    w->pvx4.release(); w->pk4.release(); w->vyz2.release(); w->rec8.release(); w->nrec8.release();
+    w->pvx4.release(); w->pk4.release(); w->vyz2.release();
     if (w->tex_vs) cudaDestroyTextureObject(w->tex_vs);
     if (w->tex_kappa) cudaDestroyTextureObject(w->tex_kappa);
     for (auto& s : w->spans) {
@@ -2014,8 +1753,6 @@ void sph_world_destroy(sph_world* w) {
         cudaEventDestroy(s.b);
     }
     if (w->h_pinned) cudaFreeHost(w->h_pinned);
-    if (w->h_ctl) cudaFreeHost(w->h_ctl);
-    w->d_ctl.release();
     w->d_ticket.release();
     w->d_nb.release();
     w->xs.release(); w->he_colors.release(); w->he_gradc.release(); w->q_out.release(); w->q_count.release();
@@ -2309,9 +2046,8 @@ static sph_status run_query(sph_world* w, AabbQuery q, const float mins[3], cons
     TRY(enter(w));
     const Consts& hc = w->hc;
     int lo[3], hi[3];
-    const int zs = hc.zsub > 0 ? hc.zsub : 1;  // the grid counts z in bins of h / zsub (and x, y in bins of h / xysub); the query box is in cells
-    const int xs = hc.xysub > 0 ? hc.xysub : 1;
-    const int go[3] = {hc.ox / xs, hc.oy / xs, hc.oz / zs}, gn[3] = {hc.nx / xs, hc.ny / xs, hc.nz / zs};
+    const int xs = hc.xysub > 0 ? hc.xysub : 1;  // the grid counts x, y in bins of h / xysub; the query box is in cells
+    const int go[3] = {hc.ox / xs, hc.oy / xs, hc.oz}, gn[3] = {hc.nx / xs, hc.ny / xs, hc.nz};
     for (int a = 0; a < 3; ++a) {  // hgrid.rs:41-52 keys, clipped IN FLOAT to the dense grid (cells outside hold nothing; +-inf / FLT_MAX bounds are legal)
         const float flo = std::floor(mins[a] / w->h), fhi = std::floor(maxs[a] / w->h);
         if (fhi < (float)go[a] || flo > (float)(go[a] + gn[a] - 1)) return SPH_OK;
@@ -2319,8 +2055,8 @@ static sph_status run_query(sph_world* w, AabbQuery q, const float mins[3], cons
         hi[a] = (int)std::fmin(fhi, (float)(go[a] + gn[a] - 1));
         if (hi[a] < lo[a]) return SPH_OK;
     }
-    q.lx = lo[0] * xs; q.ly = lo[1] * xs; q.lz = lo[2] * zs;
-    q.dx = (hi[0] - lo[0] + 1) * xs; q.dy = (hi[1] - lo[1] + 1) * xs; q.dz = (hi[2] - lo[2] + 1) * zs;
+    q.lx = lo[0] * xs; q.ly = lo[1] * xs; q.lz = lo[2];
+    q.dx = (hi[0] - lo[0] + 1) * xs; q.dy = (hi[1] - lo[1] + 1) * xs; q.dz = hi[2] - lo[2] + 1;
     for (int a = 0; a < 3; ++a) { q.mins[a] = mins[a]; q.maxs[a] = maxs[a]; }
     q.radius = w->desc.particle_radius;
     q.slot_lo = w->own_begin;
@@ -2535,14 +2271,6 @@ static sph_status slab_attach(sph_world* w, void* comm, bool own, int rank, int 
     w->desc.deterministic = 1;  // ghost-column order agreement relies on the stable in-cell order
     CU(S.d_cnt.ensure(32));
     CU(S.d_cnt64.ensure(1));
-    if (!S.comm_st) {
-        int lo_pri = 0, hi_pri = 0;
-        CU(cudaDeviceGetStreamPriorityRange(&lo_pri, &hi_pri));
-        CU(cudaStreamCreateWithPriority(&S.comm_st, cudaStreamNonBlocking, hi_pri));
-        CU(cudaEventCreateWithFlags(&S.ev_ready, cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&S.ev_done, cudaEventDisableTiming));
-    }
-    if (const char* t = getenv("SALVA_B200_SLAB_OVERLAP")) S.overlap = atoi(t) != 0;
     if (S.active) TRY(p2p_setup(w));
     return SPH_OK;
 }

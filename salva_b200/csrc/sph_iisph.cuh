@@ -41,7 +41,7 @@ k_iisph_dii(const float4* __restrict__ pos, const float4* __restrict__ vel, cons
     float rhoi = dens[i];
     float factor = -dt * dt / (rhoi * rhoi);
     float ax = 0.f, ay = 0.f, az = 0.f;
-    for_fluid_grads_pos<false>(
+    for_fluid_grads_pos(
         i, pi, L, pos, [](uint32_t) { return NoAux{}; },
         [&](uint32_t, const Pair& p, const float4& pj, NoAux) {
             float c = p.g * (pj.w * factor);
@@ -66,7 +66,7 @@ k_iisph_aii(const float4* __restrict__ pos, const float4* __restrict__ vel, cons
     float4 di = dii[i];
     float factor = dt * dt * pi.w / (rhoi * rhoi);
     float a = 0.f;
-    for_fluid_grads_pos<false>(
+    for_fluid_grads_pos(
         i, pi, L, pos, [](uint32_t) { return NoAux{}; },
         [&](uint32_t, const Pair& p, const float4& pj, NoAux) {
             float gx = p.g * p.dx, gy = p.g * p.dy, gz = p.g * p.dz;  // gradient; d_ji = gradient * factor
@@ -87,7 +87,7 @@ k_iisph_dij_pjl(const float4* __restrict__ pos, Lists L, const float* __restrict
     SPH_OWNED_INDEX(i)
     float4 pi = pos[i];
     float ax = 0.f, ay = 0.f, az = 0.f;
-    for_fluid_grads_pos<false>(
+    for_fluid_grads_pos(
         i, pi, L, pos, [&](uint32_t j) { return __ldg(&prho[j]); },
         [&](uint32_t, const Pair& p, const float4& pj, float prj) {
             float c = p.g * (-pj.w * prj);
@@ -127,7 +127,7 @@ k_iisph_next_pressures(const float4* __restrict__ pos, const float4* __restrict_
             float dji_f = dt * dt * pi.w / (rhoi * rhoi) * p_i;  // d_ji p_i = gradient * dji_f
             float derr = rho0 - pred[i];
             float sum = 0.f;
-            for_fluid_grads_pos<false>(
+            for_fluid_grads_pos(
                 i, pi, L, pos, [&](uint32_t j) { return fetch4<TEX>(s, ts, j); },
                 [&](uint32_t, const Pair& p, const float4& pj, const float4& sj) {
                     float gx = p.g * p.dx, gy = p.g * p.dy, gz = p.g * p.dz;
@@ -157,7 +157,7 @@ k_iisph_velocity_changes(const float4* __restrict__ pos, const float4* __restric
     float rho0 = C.fluids[MULTI ? fid_of(vel[i]) : 0].density0;
     float pri = prho[i];
     float ax = 0.f, ay = 0.f, az = 0.f;
-    for_fluid_grads_pos<false>(
+    for_fluid_grads_pos(
         i, pi, L, pos, [&](uint32_t j) { return __ldg(&prho[j]); },
         [&](uint32_t, const Pair& p, const float4& pj, float prj) {
             float c = p.g * (dt * pj.w * (pri + prj));

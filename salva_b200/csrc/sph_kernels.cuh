@@ -40,18 +40,14 @@ struct Consts {
     // (default, the lean path), 1 = Poly6, 2 = Spiky, 3 = Viscosity; kgen != 0 <=> any of the two is not the cubic spline
     int kw, kg, kgen;
     float poly6_n, spiky_n, visc_n;  // 315/(64 pi h^9), 15/(pi h^6), 15/(2 pi h^3)
-    int ox, oy, oz;              // grid origin in cell coordinates (one padding cell each side); oz and nz count z-BINS
+    int ox, oy, oz;              // grid origin in cell coordinates (one padding cell each side)
     int nx, ny, nz;
-    // z-bins: the counting sort splits every cell of width h into `zsub` slices along z (the run direction of the sorted
-    // order), so the neighbour search can cut each of its 9 z-runs down to the slices within reach of the particle
-    // (2h + h/zsub instead of 3h of candidates).  x and y keep the reference's cells; zsub = 1 is the plain h-cell grid.
-    int zsub;
-    float zsub_f, h_reach;       // (float)zsub; h * (1 + 1e-5): covers every |dz| the f32 test d^2 <= h^2 can accept
+    float h_reach;               // h * (1 + 1e-5): covers every |dx| the f32 test d^2 <= h^2 can accept
     // "row order" (SALVA_B200_XYSUB, one GPU, gather backend 0): x and y are binned `xysub` times finer than h (ox, oy, nx, ny then
     // count BINS), z stays the run direction.  With xysub = 2 and the usual spacing h/2 every (x, y) bin column holds ONE line of
     // particles along z, so the 32 lanes of a warp are 32 consecutive particles of a line and their k-th contacts are consecutive
     // particles of a neighbouring line: a warp-wide gather touches ~4 cache lines instead of ~17 data-pipe wavefronts
-    // (profiles/r2_l1tex_wavefront_model.md).  Contact SETS are unchanged (k_neighbors_xy clips its rows like zrun does).
+    // (profiles/r2_l1tex_wavefront_model.md).  Contact SETS are unchanged (arun clips the rows to the reference's stencil).
     int xysub;
     float xysub_f;
     int ntx, nty, ntz;           // tile grid (sph_tile.cuh): 2 x 2 cell columns x TILE_Z cells per tile
@@ -60,7 +56,6 @@ struct Consts {
                                  // two ghost columns in a multi-GPU world (x-major order keeps ghosts at both ends)
     uint32_t stride;             // neighbour-list column stride (>= n_fluid, multiple of 32)
     uint32_t cap_f, cap_b;       // list capacities (rows)
-    int use_gcache;              // gradient passes read the cached g_ij (1) or recompute it from positions (0)
     int n_fluids, n_bounds;      // object counts
     FluidParams fluids[MAX_FLUIDS];
     BoundaryParams bounds[MAX_BOUNDARIES];
@@ -75,32 +70,17 @@ __constant__ Consts C;
 __device__ __forceinline__ int cell_coord(float x) { return (int)floorf(__fdiv_rn(x, C.h)); }
 
 __device__ __forceinline__ int cell_id(int cx, int cy, int cz) { return ((cx - C.ox) * C.ny + (cy - C.oy)) * C.nz + (cz - C.oz); }
-// z-bin of a coordinate: reference cell floor(z / h) (same IEEE division) times zsub plus the slice inside the cell.  Monotone
-// non-decreasing in z (correctly rounded division, exact q - floor(q)), and every bin lies inside ONE reference cell.
-__device__ __forceinline__ int zbin(float z) {
-    const float q = __fdiv_rn(z, C.h), fl = floorf(q);
-    const int cz = (int)fl;
-    if (C.zsub == 1) return cz;
-    return cz * C.zsub + min(C.zsub - 1, (int)((q - fl) * C.zsub_f));
-}
-// Bins [lo, hi] of the z-run a particle at z (reference cell cz) has to scan: everything within h_reach of z, clipped to the
-// three reference cells cz-1..cz+1 the reference's 27-cell stencil looks at.  A pair that passes the f32 test
-// (dx^2 + dy^2) + dz^2 <= h^2 has |z_i - z_j| <= h (1 + 2^-22) < h_reach; the bounds are rounded outwards, and zbin is
-// monotone, so no accepted pair of adjacent reference cells is ever cut off: the contact sets stay exactly the reference's.
-__device__ __forceinline__ void zrun(float z, int cz, int& lo, int& hi) {
-    if (C.zsub == 1) {
-        lo = cz - 1;
-        hi = cz + 1;
-        return;
-    }
-    lo = max(zbin(__fsub_rd(z, C.h_reach)), (cz - 1) * C.zsub);
-    hi = min(zbin(__fadd_ru(z, C.h_reach)), (cz + 2) * C.zsub - 1);
-}
-// The same two functions for x / y in row order (explicit sub-division factor; zbin / zrun above are left as they were validated).
+// Row order (Consts::xysub): bin of a coordinate, reference cell floor(v / h) (same IEEE division) times `sub` plus the slice
+// inside the cell.  Monotone non-decreasing in v (correctly rounded division, exact q - floor(q)), and every bin lies inside
+// ONE reference cell.
 __device__ __forceinline__ int abin(float v, int sub, float subf) {
     const float q = __fdiv_rn(v, C.h), fl = floorf(q);
     return (int)fl * sub + min(sub - 1, (int)((q - fl) * subf));
 }
+// Bins [lo, hi] of the row a particle at v (reference cell c) has to scan: everything within h_reach of v, clipped to the three
+// reference cells c-1..c+1 the reference's 27-cell stencil looks at.  A pair that passes the f32 test d^2 <= h^2 has
+// |v_i - v_j| <= h (1 + 2^-22) < h_reach; the bounds are rounded outwards, and abin is monotone, so no accepted pair of
+// adjacent reference cells is ever cut off: the contact sets stay exactly the reference's.
 __device__ __forceinline__ void arun(float v, int c, int sub, float subf, int& lo, int& hi) {
     lo = max(abin(__fsub_rd(v, C.h_reach), sub, subf), (c - 1) * sub);
     hi = min(abin(__fadd_ru(v, C.h_reach), sub, subf), (c + 2) * sub - 1);
@@ -110,25 +90,6 @@ __device__ __forceinline__ void arun(float v, int c, int sub, float subf, int& l
 __device__ __forceinline__ float dist2_exact(float dx, float dy, float dz) {
     return __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
 }
-// The same value, bit for bit, with the x and y lanes done by Blackwell's packed-f32 instructions (FADD2 / FMUL2: two IEEE
-// round-to-nearest operations per issue slot; sm_100+).  Only subtract and multiply are packed: ptxas contracts a packed
-// multiply feeding a packed add into FFMA2 even with explicit .rn, which would change the rounding; the adds stay scalar.
-// (Experiment only, see SPH_PACKED_F32 at scan_run: fewer issue slots, but not faster.)
-__device__ __forceinline__ unsigned long long pack_f32x2(float a, float b) {
-    unsigned long long r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(a), "f"(b));
-    return r;
-}
-__device__ __forceinline__ float dist2_exact_packed(unsigned long long pi_xy, float pi_z, const float4& pj) {
-    unsigned long long d;
-    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(pi_xy), "l"(pack_f32x2(pj.x, pj.y)));
-    asm("mul.rn.f32x2 %0, %1, %1;" : "=l"(d) : "l"(d));
-    float sx, sy;
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(sx), "=f"(sy) : "l"(d));
-    const float dz = __fsub_rn(pi_z, pj.z);
-    return __fadd_rn(__fadd_rn(sx, sy), __fmul_rn(dz, dz));
-}
-
 // cubic_spline_kernel.rs:12-33: W(r) for q = r/h.
 __device__ __forceinline__ float kernel_w(float r) {
     float q = r * C.inv_h;
@@ -139,21 +100,6 @@ __device__ __forceinline__ float kernel_w(float r) {
     float rhs = q <= 0.5f ? a : (q <= 1.0f ? b : 0.0f);
     return C.sigma * rhs;
 }
-// cubic_spline_kernel.rs:55-80 + kernel.rs:18-24: returns g with grad W_ij = g * (x_i - x_j);
-// zero if |x_ij|^2 <= eps^2, q <= 1e-5 or q > 1.
-__device__ __forceinline__ float kernel_gfac(float d2, float r, float inv_r) {
-    float q = r * C.inv_h;
-    float t = 1.0f - q;
-    float a = (q * 3.0f - 2.0f) * q * 6.0f;
-    float b = -t * t * 6.0f;
-    float rhs = q <= 0.5f ? a : b;
-    bool zero = (q > 1.0f) | (q <= 1.0e-5f) | !(d2 > F32_EPS * F32_EPS);
-    return zero ? 0.0f : C.dsigma * rhs * inv_r;
-}
-
-#ifndef SPH_FAST_PAIR
-#define SPH_FAST_PAIR 1
-#endif
 // MUFU.RSQ without the denormal-rescue sequence rsqrtf() compiles to (3 extra instructions per contact): operands
 // here are squared distances >= g_t2 ~ 1e-14 or exactly 0 (self contact: +inf, masked by the d2 > g_t2 select).
 __device__ __forceinline__ float rsqrt_ftz(float x) {
@@ -240,8 +186,7 @@ __device__ __forceinline__ Pair make_pair(const float4& pi, const float4& pj) {
         p.g = o.y;
         return p;
     }
-#if SPH_FAST_PAIR
-    // Lean evaluation (about half the instructions of the guarded one below): contacts come from lists built with
+    // Lean evaluation (about half the instructions of a guarded rsqrtf one): contacts come from lists built with
     // d^2 <= h^2, so q <= 1 up to rounding (where (1 - q)^2 ~ 1e-14 anyway), and the two "zero gradient" guards of the
     // reference (|x_ij|^2 > eps^2, q > 1e-5) collapse into one select on d2.  d2 == 0 gives inv_r = +inf and NaNs in
     // r / q, all discarded by the selects (never multiplied).
@@ -266,12 +211,6 @@ __device__ __forceinline__ Pair make_pair(const float4& pi, const float4& pj) {
     } else {
         p.g = 0.f;
     }
-#else
-    float inv_r = rsqrtf(fmaxf(p.d2, 1.0e-30f));
-    p.r = p.d2 * inv_r;
-    p.w = NEED_W ? kernel_w(p.r) : 0.f;
-    p.g = NEED_G ? kernel_gfac(p.d2, p.r, inv_r) : 0.f;
-#endif
     return p;
 }
 
@@ -377,7 +316,7 @@ __global__ void k_cell_hist(const float4* __restrict__ pos, uint32_t n, uint32_t
         return;
     }
     float4 p = pos[i];
-    uint32_t id = (uint32_t)cell_id(cell_coord(p.x), cell_coord(p.y), zbin(p.z));
+    uint32_t id = (uint32_t)cell_id(cell_coord(p.x), cell_coord(p.y), cell_coord(p.z));
     cid[i] = id;
     rank[i] = atomicAdd(&count[id], 1u);
 }
@@ -388,7 +327,7 @@ __global__ void k_cell_hist_xy(const float4* __restrict__ pos, uint32_t n, uint3
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     float4 p = pos[i];
-    uint32_t id = (uint32_t)cell_id(abin(p.x, C.xysub, C.xysub_f), abin(p.y, C.xysub, C.xysub_f), zbin(p.z));
+    uint32_t id = (uint32_t)cell_id(abin(p.x, C.xysub, C.xysub_f), abin(p.y, C.xysub, C.xysub_f), cell_coord(p.z));
     cid[i] = id;
     rank[i] = atomicAdd(&count[id], 1u);
 }
@@ -571,53 +510,15 @@ __global__ void k_scanK_add(ScanSet<K> io, uint32_t n, ScanSet<K> block_offsets)
 // only records hits in a 32-bit mask per chunk of 32 candidates; the (short) emit loop then walks the set bits in
 // ascending order, which keeps every list in the same order as a plain scan.
 // ------------------------------------------------------------------------------------------------
-// TEX (optional): a texture over the same array P; odd candidates are then fetched through the texture pipe, so the candidate
-// stream (243 loads per particle) is split over both L1TEX front ends like the gather passes' (SALVA_B200_NBR_TEX).
-// Packed-f32 candidate test (FADD2 / FMUL2, below): bit-identical contact sets (all GPU tests pass with it) and 9.75 instead of
-// 12.75 issue slots per candidate in SASS, but measured SLOWER (k_neighbors 1.637 -> 1.669 ms at C3, 0.662 -> 0.683 ms on the C4
-// slice, profiles/r2_exp_m_raw.txt): the packed instructions do not issue at the scalar rate and the LSU data pipe (78 %) is the
-// co-limiter anyway.  Kept behind -DSPH_PACKED_F32=1.
-#ifndef SPH_PACKED_F32
-#define SPH_PACKED_F32 0
-#endif
-template <bool NTEX = false, class Accept, class Emit>
-__device__ __forceinline__ void scan_run(const float4& pi, const float4* __restrict__ P, uint32_t s, uint32_t e, Accept accept, Emit emit,
-                                         cudaTextureObject_t TEX = 0) {
+template <class Accept, class Emit>
+__device__ __forceinline__ void scan_run(const float4& pi, const float4* __restrict__ P, uint32_t s, uint32_t e, Accept accept, Emit emit) {
     for (uint32_t base = s; base < e; base += 32u) {
         const uint32_t n = min(32u, e - base);
         const float4* __restrict__ q = P + base;
         uint32_t rej = 0u;  // candidate t of the chunk ends up in bit n - 1 - t; set = rejected
-        uint32_t t = 0;
-#if SPH_PACKED_F32
-        if (!NTEX) {
-            // two candidates per trip: x/y differences and squares, the two z squares and the two (h^2 - d^2) as packed pairs;
-            // 9.5 issue slots per candidate instead of 12.75 (SASS: 2 FADD2 + 3 FMUL2 + 1 FADD2 + 6 FADD + 2 SHF + 2 LDG per pair)
-            const unsigned long long pi_xy = pack_f32x2(pi.x, pi.y), hh = pack_f32x2(C.h2, C.h2);
-#pragma unroll 2
-            for (; t + 1 < n; t += 2) {
-                const float4 pa = __ldg(&q[t]), pb = __ldg(&q[t + 1]);
-                unsigned long long da, db, dz, r;
-                asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(da) : "l"(pi_xy), "l"(pack_f32x2(pa.x, pa.y)));
-                asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(db) : "l"(pi_xy), "l"(pack_f32x2(pb.x, pb.y)));
-                asm("mul.rn.f32x2 %0, %1, %1;" : "=l"(da) : "l"(da));
-                asm("mul.rn.f32x2 %0, %1, %1;" : "=l"(db) : "l"(db));
-                dz = pack_f32x2(__fsub_rn(pi.z, pa.z), __fsub_rn(pi.z, pb.z));
-                asm("mul.rn.f32x2 %0, %1, %1;" : "=l"(dz) : "l"(dz));
-                float ax, ay, bx, by, za, zb, r0, r1;
-                asm("mov.b64 {%0, %1}, %2;" : "=f"(ax), "=f"(ay) : "l"(da));
-                asm("mov.b64 {%0, %1}, %2;" : "=f"(bx), "=f"(by) : "l"(db));
-                asm("mov.b64 {%0, %1}, %2;" : "=f"(za), "=f"(zb) : "l"(dz));
-                const float d2a = __fadd_rn(__fadd_rn(ax, ay), za), d2b = __fadd_rn(__fadd_rn(bx, by), zb);  // scalar adds: see dist2_exact_packed
-                asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(hh), "l"(pack_f32x2(d2a, d2b)));
-                asm("mov.b64 {%0, %1}, %2;" : "=f"(r0), "=f"(r1) : "l"(r));
-                rej = __funnelshift_l(__float_as_uint(r0), rej, 1);
-                rej = __funnelshift_l(__float_as_uint(r1), rej, 1);
-            }
-        }
-#endif
 #pragma unroll 4
-        for (; t < n; ++t) {
-            const float4 pj = (NTEX && (t & 1u)) ? tex1Dfetch<float4>(TEX, (int)(base + t)) : __ldg(&q[t]);
+        for (uint32_t t = 0; t < n; ++t) {
+            const float4 pj = __ldg(&q[t]);
             const float d2 = dist2_exact(pi.x - pj.x, pi.y - pj.y, pi.z - pj.z);
             // d2 <= h*h  <=>  the sign bit of (h*h - d2) is clear (a float difference is zero only for equal operands;
             // NaN positions never get here, k_bounds rejects them): shift that bit into the mask with one funnel shift
@@ -633,15 +534,14 @@ __device__ __forceinline__ void scan_run(const float4& pi, const float4* __restr
     }
 }
 
-#ifndef SPH_NBR_RUNPTR
-#define SPH_NBR_RUNPTR 1  // list entries addressed with a running pointer instead of recomputing ((k >> 2) * stride + i) * 4 + (k & 3)
-#endif
-template <bool MULTI, bool NTEX>
-__global__ void __launch_bounds__(128)
+// Minimum blocks per SM: left to itself ptxas gives these kernels 40 registers and spills a cell coordinate across the slow
+// path of the IEEE division in cell_coord(); the bounds below keep every instantiation spill-free at no higher register count.
+template <bool MULTI>
+__global__ void __launch_bounds__(128, MULTI ? 12 : 10)
 k_neighbors(const float4* __restrict__ pos, const float4* __restrict__ vel, const uint32_t* __restrict__ cstart,
             const float4* __restrict__ bpos, const float4* __restrict__ bvel, const uint32_t* __restrict__ bstart,
             uint32_t* __restrict__ nbr_f, uint32_t* __restrict__ nbr_b, uint32_t* __restrict__ cnt_f, uint32_t* __restrict__ cnt_b,
-            uint32_t* __restrict__ maxcnt /* [0]=fluid,[1]=boundary */, cudaTextureObject_t tpos) {
+            uint32_t* __restrict__ maxcnt /* [0]=fluid,[1]=boundary */) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     uint32_t nf = 0, nb = 0;
     const bool owned = i < C.n_owned;
@@ -650,14 +550,14 @@ k_neighbors(const float4* __restrict__ pos, const float4* __restrict__ vel, cons
         float4 pi = pos[i];
         uint32_t fi = MULTI ? fid_of(vel[i]) : 0u;
         int cx = cell_coord(pi.x), cy = cell_coord(pi.y), cz = cell_coord(pi.z);
-        int zlo, zhi;
-        zrun(pi.z, cz, zlo, zhi);
+        const int zlo = cz - 1, zhi = cz + 1;
+        // entry k of particle i lives at ((k >> 2) * stride + i) * 4 + (k & 3): walked with a running pointer
         uint32_t* wp = nbr_f + (size_t)i * 4;                  // slot 0 of group 0 of this particle's column
         const size_t gstep = (size_t)C.stride * 4 - 4;         // from behind slot 3 of a group to slot 0 of the next one
         for (int ax = -1; ax <= 1; ++ax)
             for (int ay = -1; ay <= 1; ++ay) {
                 const int lo = cell_id(cx + ax, cy + ay, zlo), hi = lo + (zhi - zlo) + 1;
-                scan_run<NTEX>(
+                scan_run(
                     pi, pos, cstart[lo], cstart[hi],
                     [&](uint32_t j) {
                         if (!MULTI) return true;
@@ -667,18 +567,11 @@ k_neighbors(const float4* __restrict__ pos, const float4* __restrict__ vel, cons
                     [&](uint32_t j) {
                         // (one 4-byte store per hit: collecting four hits in registers and storing 16-byte groups was measured
                         //  SLOWER, 1.66 -> 1.80 ms at C3 — the shift-in costs more issue slots than the stores save)
-                        //  entry k of particle i lives at ((k >> 2) * stride + i) * 4 + (k & 3): walked with a running pointer)
-#if SPH_NBR_RUNPTR
                         if (nf < C.cap_f) *wp = j;
                         ++nf;
                         ++wp;
                         if ((nf & 3u) == 0u) wp += gstep;
-#else
-                        if (nf < C.cap_f) nbr_f[((size_t)(nf >> 2) * C.stride + i) * 4 + (nf & 3)] = j;
-                        ++nf;
-#endif
-                    },
-                    tpos);
+                    });
                 if (C.n_bound)
                     scan_run(
                         pi, bpos, bstart[lo], bstart[hi],
@@ -691,11 +584,7 @@ k_neighbors(const float4* __restrict__ pos, const float4* __restrict__ vel, cons
                             ++nb;
                         });
             }
-#if SPH_NBR_RUNPTR
         for (uint32_t t = nf; t < ((nf + 3u) & ~3u) && t < C.cap_f; ++t) *wp++ = i;  // pad the last group
-#else
-        for (uint32_t t = nf; t < ((nf + 3u) & ~3u) && t < C.cap_f; ++t) nbr_f[((size_t)(t >> 2) * C.stride + i) * 4 + (t & 3)] = i;
-#endif
         cnt_f[i] = nf;
         cnt_b[i] = nb;
     }
@@ -711,10 +600,10 @@ k_neighbors(const float4* __restrict__ pos, const float4* __restrict__ vel, cons
 }
 
 // Row order (Consts::xysub > 1): the same search over the bin rows within reach in x and y (5 x 5 rows of width h / 2 at xysub = 2
-// instead of 3 x 3 of width h; arun() clips exactly like zrun(), so the contact sets are the reference's).  A separate kernel so that
+// instead of 3 x 3 of width h; arun() clips to the reference's stencil, so the contact sets are the reference's).  A separate kernel so that
 // the default path above stays byte for byte what was validated.
 template <bool MULTI>
-__global__ void __launch_bounds__(128)
+__global__ void __launch_bounds__(128, MULTI ? 0 : 10)  // (see k_neighbors; 0: no minimum)
 k_neighbors_xy(const float4* __restrict__ pos, const float4* __restrict__ vel, const uint32_t* __restrict__ cstart,
                const float4* __restrict__ bpos, const float4* __restrict__ bvel, const uint32_t* __restrict__ bstart,
                uint32_t* __restrict__ nbr_f, uint32_t* __restrict__ nbr_b, uint32_t* __restrict__ cnt_f, uint32_t* __restrict__ cnt_b,
@@ -727,16 +616,16 @@ k_neighbors_xy(const float4* __restrict__ pos, const float4* __restrict__ vel, c
         float4 pi = pos[i];
         uint32_t fi = MULTI ? fid_of(vel[i]) : 0u;
         const int cx = cell_coord(pi.x), cy = cell_coord(pi.y), cz = cell_coord(pi.z);
-        int xlo, xhi, ylo, yhi, zlo, zhi;
+        int xlo, xhi, ylo, yhi;
         arun(pi.x, cx, C.xysub, C.xysub_f, xlo, xhi);
         arun(pi.y, cy, C.xysub, C.xysub_f, ylo, yhi);
-        zrun(pi.z, cz, zlo, zhi);
+        const int zlo = cz - 1, zhi = cz + 1;
         uint32_t* wp = nbr_f + (size_t)i * 4;
         const size_t gstep = (size_t)C.stride * 4 - 4;
         for (int bx = xlo; bx <= xhi; ++bx)
             for (int by = ylo; by <= yhi; ++by) {
                 const int lo = cell_id(bx, by, zlo), hi = lo + (zhi - zlo) + 1;
-                scan_run<false>(
+                scan_run(
                     pi, pos, cstart[lo], cstart[hi],
                     [&](uint32_t j) {
                         if (!MULTI) return true;
@@ -788,8 +677,8 @@ k_boundary_volumes_xy(const float4* __restrict__ bpos, const float4* __restrict_
         float den = 0.f;
         for (int bx = (cx - 1) * C.xysub; bx < (cx + 2) * C.xysub; ++bx)
             for (int by = (cy - 1) * C.xysub; by < (cy + 2) * C.xysub; ++by) {
-                const int base = cell_id(bx, by, (cz - 1) * C.zsub);
-                const uint32_t s = bstart[base], e = bstart[base + 3 * C.zsub];
+                const int base = cell_id(bx, by, cz - 1);
+                const uint32_t s = bstart[base], e = bstart[base + 3];
                 for (uint32_t j = s; j < e; ++j) {
                     float4 pj = __ldg(&bpos[j]);
                     float dx = pi.x - pj.x, dy = pi.y - pj.y, dz = pi.z - pj.z;
@@ -824,8 +713,8 @@ k_boundary_volumes(const float4* __restrict__ bpos, const float4* __restrict__ b
         float den = 0.f;
         for (int ax = -1; ax <= 1; ++ax)
             for (int ay = -1; ay <= 1; ++ay) {
-                int base = cell_id(cx + ax, cy + ay, (cz - 1) * C.zsub);  // all bins of the three reference cells cz-1..cz+1
-                uint32_t s = bstart[base], e = bstart[base + 3 * C.zsub];
+                int base = cell_id(cx + ax, cy + ay, cz - 1);  // the three cells cz-1..cz+1
+                uint32_t s = bstart[base], e = bstart[base + 3];
                 for (uint32_t j = s; j < e; ++j) {
                     float4 pj = __ldg(&bpos[j]);
                     float dx = pi.x - pj.x, dy = pi.y - pj.y, dz = pi.z - pj.z;
@@ -875,60 +764,10 @@ __global__ void k_reduce_partials(const float* __restrict__ partial, uint32_t nb
 #endif
 constexpr int PASS_T = SPH_PASS_T;  // threads per block of the gather passes
 
-// Device-side control of the Jacobi loops (`for i in 0..max { eval; if err <= tol && i >= min { break } update }`,
-// dfsph_solver.rs:439-463,474-502).  The host enqueues a few iterations ahead; k_loop_decide takes the reference's
-// break decision on the device and the evaluation / update kernels of iterations that must not run exit immediately
-// (`active` gates evaluations, `do_update` gates updates).  One host sync per loop instead of one per evaluation.
-struct LoopCtl {
-    int active;       // further evaluations may run
-    int do_update;    // the update following the last evaluation must run
-    uint32_t iter;    // updates decided so far
-    uint32_t n_eval;  // evaluations executed
-    float last_err;
-    float tol;
-    uint32_t min_iter, max_iter;
-    int forced;       // >= 0: run exactly this many updates (parity aid), ignore the error
-    int n_fluids;
-    float inv_count[MAX_FLUIDS];  // 1 / particle count per fluid (global count in a slab world); 0 for empty fluids
-};
-__global__ void k_loop_decide(LoopCtl* __restrict__ ctl, const float* __restrict__ errsum) {
-    if (threadIdx.x != 0 || blockIdx.x != 0) return;
-    if (!ctl->active) {
-        ctl->do_update = 0;
-        return;
-    }
-    ctl->n_eval++;
-    float err = 0.f;
-    for (int f = 0; f < ctl->n_fluids; ++f) err = fmaxf(err, errsum[f] * ctl->inv_count[f]);  // per-fluid mean, max over fluids
-    ctl->last_err = err;
-    bool stop = ctl->forced >= 0 ? (int)ctl->iter >= ctl->forced : (err <= ctl->tol && ctl->iter >= ctl->min_iter);
-    if (stop) {
-        ctl->active = 0;
-        ctl->do_update = 0;
-    } else {
-        ctl->do_update = 1;
-        ctl->iter++;
-        if (ctl->iter >= ctl->max_iter) ctl->active = 0;  // the loop ends after this update without another evaluation
-    }
-}
-
-struct __align__(32) Rec8 {
-    float x, y, z, vx, vy, vz, rho, pad;
-};
-__device__ __forceinline__ void ld_rec8(const Rec8* __restrict__ p, float4& a, float4& b) {
-    asm("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-        : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w), "=f"(b.x), "=f"(b.y), "=f"(b.z), "=f"(b.w)
-        : "l"(p));
-}
-__device__ __forceinline__ void st_rec8(Rec8* p, float x, float y, float z, float vx, float vy, float vz, float rho) {
-    asm volatile("st.global.v8.f32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "f"(x), "f"(y), "f"(z), "f"(vx), "f"(vy), "f"(vz), "f"(rho), "f"(0.f)
-                 : "memory");
-}
-
 // The fluid reorder fused with k_make_vstar: the sorted pos / vel / vc are in registers anyway, so v* = vel + vc and the packed
 // gather records are written by the same pass (saves re-reading 48 B per particle and a launch).  g.in4 / out4 [0..2] = pos, vel, vc.
 __global__ void k_gather_vstar(uint32_t n, const uint32_t* __restrict__ perm, GatherSet g, float4* __restrict__ vs, float4* __restrict__ pvx,
-                               float2* __restrict__ vyz, Rec8* __restrict__ rec) {
+                               float2* __restrict__ vyz) {
     uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n) return;
     const uint32_t src = perm[s];
@@ -941,9 +780,7 @@ __global__ void k_gather_vstar(uint32_t n, const uint32_t* __restrict__ perm, Ga
         if (a < g.n1) g.out1[a][s] = g.in1[a][src];
     const float sx = v.x + c.x, sy = v.y + c.y, sz = v.z + c.z;
     vs[s] = make_float4(sx, sy, sz, 0.f);
-    if (rec) {
-        st_rec8(rec + s, p.x, p.y, p.z, sx, sy, sz, 0.f);
-    } else if (pvx) {
+    if (pvx) {
         pvx[s] = make_float4(p.x, p.y, p.z, sx);
         vyz[s] = make_float2(sy, sz);
     }
@@ -951,16 +788,13 @@ __global__ void k_gather_vstar(uint32_t n, const uint32_t* __restrict__ perm, Ga
 
 // v* = vel + vc after the reorder (the divergence solve works on vel + vc carried over from the previous step, Appendix A.3.2)
 __global__ void k_make_vstar(const float4* __restrict__ vel, const float4* __restrict__ vc, float4* __restrict__ vs, const float4* __restrict__ pos,
-                             float4* __restrict__ pvx, float2* __restrict__ vyz, Rec8* __restrict__ rec) {
+                             float4* __restrict__ pvx, float2* __restrict__ vyz) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= C.n_fluid) return;
     float4 v = vel[i], c = vc[i];
     float sx = v.x + c.x, sy = v.y + c.y, sz = v.z + c.z;
     vs[i] = make_float4(sx, sy, sz, 0.f);
-    if (rec) {  // 256-bit gather records; rho is filled in by the first velocity update of the step
-        float4 p = pos[i];
-        st_rec8(rec + i, p.x, p.y, p.z, sx, sy, sz, 0.f);
-    } else if (pvx) {  // uniform-mass packed records (sph_passes.cuh)
+    if (pvx) {  // uniform-mass packed records (sph_passes.cuh)
         float4 p = pos[i];
         pvx[i] = make_float4(p.x, p.y, p.z, sx);
         vyz[i] = make_float2(sy, sz);
@@ -1032,18 +866,14 @@ __global__ void k_set_gravity(const float4* __restrict__ vel, float4* __restrict
 // the next step's k_fold_velocities / k_set_gravity overwrites them with gravity before any force adds to them, so the
 // array doubles as the SPH_DBG_ACCELERATION view and the pass saves 32 B per particle of stores.
 __global__ void k_integrate_acc(const float4* __restrict__ vel, float4* __restrict__ vc, float4* __restrict__ vs, const float4* __restrict__ acc, float dt,
-                                float4* __restrict__ pvx, float2* __restrict__ vyz, const float4* __restrict__ pos, Rec8* __restrict__ rec,
-                                const float* __restrict__ dens) {
+                                float4* __restrict__ pvx, float2* __restrict__ vyz) {
     SPH_OWNED_INDEX(i)
     float4 a = acc[i], c = vc[i], v = vel[i];
     c.x += a.x * dt; c.y += a.y * dt; c.z += a.z * dt;
     vc[i] = c;
     float sx = v.x + c.x, sy = v.y + c.y, sz = v.z + c.z;
     vs[i] = make_float4(sx, sy, sz, 0.f);
-    if (rec) {
-        const float4 p = pos[i];
-        st_rec8(rec + i, p.x, p.y, p.z, sx, sy, sz, dens[i]);
-    } else if (pvx) {
+    if (pvx) {
         pvx[i].w = sx;  // xyz already hold the position
         vyz[i] = make_float2(sy, sz);
     }

@@ -19,8 +19,6 @@ struct Lists {
     const uint32_t* nbr_b;  // nbr_b[k * stride + i]
     const uint32_t* cnt_f;
     const uint32_t* cnt_b;
-    const float4* g_f;      // g_f[(k / 4) * stride + i]: cached gradient scalars g_ij = W'(|x_ij|) / |x_ij| of the same 4 contacts
-                            // (contact.gradient = g * x_ij, helper.rs:24-25); written by k_density_alpha once per step, 0 in tail slots
 };
 
 struct NoAux {};
@@ -35,31 +33,14 @@ __device__ __forceinline__ auto call_gather(F& f, uint32_t j, int u) {
     else return f(j);
 }
 
-// Slot range a launch covers.  One launch normally covers all owned slots; a slab world splits the Jacobi-loop kernels
-// into [boundary columns] + [interior] so the ghost exchange of the boundary columns overlaps the interior launch.
+// Slot range a launch covers: the owned slots [begin, begin + count).
 struct Range {
     uint32_t begin, count;
 };
 
 // The contact lists are streamed exactly once per pass: load them with the evict-first policy so they do not push the
-// gathered particle data out of L1/L2, and pull the rows a few groups ahead into L2 (each group row of a warp is a
-// separate 512-byte segment `stride` elements apart, which no hardware prefetcher follows).
-#ifndef SPH_LIST_PREFETCH
-#define SPH_LIST_PREFETCH 0
-#endif
-// Cached gradient scalars (g_f): measured slower in rounds 1 and 2 (profiles/r2_exp_a_variants.md) and, worse, the runtime
-// switch between the cached and the recomputed path sits inside the 4-way unrolled contact loops, where a uniform branch
-// costs ~10 % (k_vel_update_u 0.0653 ms with it vs 0.0578 ms without, C2).  Compiled out unless -DSPH_GCACHE=1.
-#ifndef SPH_GCACHE
-#define SPH_GCACHE 0
-#endif
+// gathered particle data out of L1/L2.
 __device__ __forceinline__ uint4 ld_list(const uint4* p) { return __ldcs(p); }
-__device__ __forceinline__ float4 ld_list(const float4* p) { return __ldcs(p); }
-__device__ __forceinline__ void prefetch_list(const void* p) {
-#if SPH_LIST_PREFETCH > 0
-    asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
-#endif
-}
 
 // ldpos(j) -> float4 whose xyz is the neighbour position (w = whatever the array packs there); ld(j) -> Aux loads
 // whatever else the pass needs from neighbour j; ff(j, pair, posrec_j, aux) consumes one contact.
@@ -72,7 +53,6 @@ __device__ __forceinline__ void for_fluid_contacts_g(uint32_t i, const float4& p
     for (uint32_t q = 0; q < nq; ++q) {
         uint4 Jn = J;
         if (q + 1 < nq) Jn = ld_list(col + (size_t)(q + 1) * C.stride);  // fetch the next group of indices early
-        if (q + 1 + SPH_LIST_PREFETCH < nq) prefetch_list(col + (size_t)(q + 1 + SPH_LIST_PREFETCH) * C.stride);
         uint32_t j[4] = {J.x, J.y, J.z, J.w};
         const uint32_t k0 = q * 4u;
         bool ok[4];
@@ -101,30 +81,18 @@ __device__ __forceinline__ void for_fluid_contacts_g(uint32_t i, const float4& p
 // gathers are issued back to back before any arithmetic, and the next group's list indices are prefetched.
 // (A deeper software pipeline — gathers one group ahead — was measured SLOWER: 80-96 registers halve the occupancy,
 // C2 predicted-density pass 0.127 ms vs 0.099 ms; profiles/r1_v1_batching_tex_c2.md.)
-// C.use_gcache selects where the gradient scalar g_ij = W'(|x_ij|)/|x_ij| comes from: the per-step cache written by
-// k_density_alpha (fewer instructions, +4 B/contact of traffic; measured neutral at 1M, slower at 10M where the list
-// traffic already puts DRAM at ~50 %) or recomputed from the positions (default).
-// No tail masking: padded slots are (j = i, g = 0) and a self contact has zero gradient either way.
-template <bool NEED_D2, bool NEED_W = false, class LP, class LD, class FF>
+// No tail masking: padded slots are (j = i) and a self contact has zero gradient.
+template <bool NEED_W = false, class LP, class LD, class FF>
 __device__ __forceinline__ void for_fluid_grads(uint32_t i, const float4& pi, const Lists& L, LP ldpos, LD ld, FF ff) {
     const uint32_t n = min(L.cnt_f[i], C.cap_f);
     const uint32_t nq = (n + 3u) >> 2;
     if (nq == 0) return;
-    const bool cached = SPH_GCACHE && C.use_gcache != 0;  // compile-time off: the uniform branch inside the unrolled group costs ~10 % of a pass
     const uint4* col = L.nbr_f + i;
-    const float4* gcol = L.g_f + i;
     uint4 J = ld_list(col);
-    float4 Gq = cached ? ld_list(gcol) : make_float4(0.f, 0.f, 0.f, 0.f);
     for (uint32_t q = 0; q < nq; ++q) {
         uint4 Jn = J;
-        float4 Gn = Gq;
-        if (q + 1 < nq) {  // fetch the next group early
-            Jn = ld_list(col + (size_t)(q + 1) * C.stride);
-            if (cached) Gn = ld_list(gcol + (size_t)(q + 1) * C.stride);
-        }
-        if (q + 1 + SPH_LIST_PREFETCH < nq) prefetch_list(col + (size_t)(q + 1 + SPH_LIST_PREFETCH) * C.stride);
+        if (q + 1 < nq) Jn = ld_list(col + (size_t)(q + 1) * C.stride);  // fetch the next group early
         const uint32_t j[4] = {J.x, J.y, J.z, J.w};
-        const float g[4] = {Gq.x, Gq.y, Gq.z, Gq.w};
         float4 pj[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) pj[u] = call_gather(ldpos, j[u], u);
@@ -133,25 +101,15 @@ __device__ __forceinline__ void for_fluid_grads(uint32_t i, const float4& pi, co
         for (int u = 0; u < 4; ++u) aux[u] = call_gather(ld, j[u], u);
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
-            Pair p;
-            if (cached) {
-                p.dx = pi.x - pj[u].x;
-                p.dy = pi.y - pj[u].y;
-                p.dz = pi.z - pj[u].z;
-                p.g = g[u];
-                if (NEED_D2) p.d2 = fmaf(p.dz, p.dz, fmaf(p.dy, p.dy, p.dx * p.dx));
-            } else {
-                p = make_pair<NEED_W, true>(pi, pj[u]);
-            }
+            Pair p = make_pair<NEED_W, true>(pi, pj[u]);
             ff(j[u], p, pj[u], aux[u]);
         }
         J = Jn;
-        Gq = Gn;
     }
 }
-template <bool NEED_D2, class LD, class FF>
+template <class LD, class FF>
 __device__ __forceinline__ void for_fluid_grads_pos(uint32_t i, const float4& pi, const Lists& L, const float4* __restrict__ pos, LD ld, FF ff) {
-    for_fluid_grads<NEED_D2>(i, pi, L, [&](uint32_t j) { return __ldg(&pos[j]); }, ld, ff);
+    for_fluid_grads(i, pi, L, [&](uint32_t j) { return __ldg(&pos[j]); }, ld, ff);
 }
 
 template <bool W, bool G, class LD, class FF>
@@ -220,7 +178,7 @@ __device__ __forceinline__ void reduce_error(float e, uint32_t fi, bool valid, f
 // ------------------------------------------------------------------------------------------------
 template <bool MULTI>
 __global__ void __launch_bounds__(PASS_T, SPH_PASS_MINB)
-k_density_alpha(const float4* __restrict__ pos, const float4* __restrict__ vel, const float4* __restrict__ bpos, Lists L, float4* __restrict__ g_out,
+k_density_alpha(const float4* __restrict__ pos, const float4* __restrict__ vel, const float4* __restrict__ bpos, Lists L,
                 float* __restrict__ dens, float* __restrict__ alpha, int* __restrict__ err) {
     SPH_OWNED_INDEX(i)
     float4 pi = pos[i];
@@ -234,17 +192,14 @@ k_density_alpha(const float4* __restrict__ pos, const float4* __restrict__ vel, 
         for (uint32_t q = 0; q < nq; ++q) {
             uint4 Jn = J;
             if (q + 1 < nq) Jn = ld_list(col + (size_t)(q + 1) * C.stride);
-            if (q + 1 + SPH_LIST_PREFETCH < nq) prefetch_list(col + (size_t)(q + 1 + SPH_LIST_PREFETCH) * C.stride);
             const uint32_t j[4] = {J.x, J.y, J.z, J.w};
             float4 pj[4];
 #pragma unroll
             for (int u = 0; u < 4; ++u) pj[u] = __ldg(&pos[j[u]]);  // tail slots point at i itself
-            float g[4];
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 const bool ok = q * 4u + u < n;
                 Pair p = make_pair<true, true>(pi, pj[u]);
-                g[u] = ok ? p.g : 0.f;
                 if (ok) {
                     rho = fmaf(pj[u].w, p.w, rho);
                     float s = p.g * pj[u].w;  // m_j * gradient
@@ -253,7 +208,6 @@ k_density_alpha(const float4* __restrict__ pos, const float4* __restrict__ vel, 
                     gx += ax; gy += ay; gz += az;
                 }
             }
-            if (SPH_GCACHE && C.use_gcache) g_out[(size_t)q * C.stride + i] = make_float4(g[0], g[1], g[2], g[3]);  // helper.rs:24-25, cached for the step
             J = Jn;
         }
     }
@@ -285,7 +239,7 @@ template <bool MULTI, bool UNI>
 __global__ void __launch_bounds__(PASS_T, SPH_PASS_MINB)
 k_density_alpha_div(const float4* __restrict__ posrec /* pos4 or pvx4 */, cudaTextureObject_t tposrec, const float4* __restrict__ vs, cudaTextureObject_t tvs,
                     const float2* __restrict__ vyz, cudaTextureObject_t tvyz, const float4* __restrict__ vel, const float4* __restrict__ bpos, Lists L,
-                    float4* __restrict__ g_out, float* __restrict__ dens, float* __restrict__ alpha, float* __restrict__ divv, float* __restrict__ kappa,
+                    float* __restrict__ dens, float* __restrict__ alpha, float* __restrict__ divv, float* __restrict__ kappa,
                     float4* __restrict__ pk4, float* __restrict__ partial, int* __restrict__ err, uint32_t* __restrict__ ticket,
                     float* __restrict__ errsum, Range rg) {
     __shared__ float sm[32];
@@ -316,7 +270,6 @@ k_density_alpha_div(const float4* __restrict__ posrec /* pos4 or pvx4 */, cudaTe
         for (uint32_t q = 0; q < nq; ++q) {
             uint4 Jn = J;
             if (q + 1 < nq) Jn = ld_list(col + (size_t)(q + 1) * C.stride);
-            if (q + 1 + SPH_LIST_PREFETCH < nq) prefetch_list(col + (size_t)(q + 1 + SPH_LIST_PREFETCH) * C.stride);
             const uint32_t j[4] = {J.x, J.y, J.z, J.w};
             float4 pj[4];
             Vel3 vj[4];
@@ -332,12 +285,10 @@ k_density_alpha_div(const float4* __restrict__ posrec /* pos4 or pvx4 */, cudaTe
                     vj[u] = Vel3{s.x, s.y, s.z};
                 }
             }
-            float g[4];
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 const bool ok = q * 4u + u < n;
                 Pair p = make_pair<true, true>(pi, pj[u]);
-                g[u] = ok ? p.g : 0.f;
                 if (ok) {
                     const float mj = UNI ? umass : pj[u].w;
                     rho = fmaf(mj, p.w, rho);
@@ -349,7 +300,6 @@ k_density_alpha_div(const float4* __restrict__ posrec /* pos4 or pvx4 */, cudaTe
                     d = fmaf(dv * p.g, mj, d);
                 }
             }
-            if (SPH_GCACHE && C.use_gcache) g_out[(size_t)q * C.stride + i] = make_float4(g[0], g[1], g[2], g[3]);
             J = Jn;
         }
         for_boundary_contacts<true, true>(i, pi, L, bpos, [&](uint32_t, const Pair& p, const float4& pj) {
@@ -383,13 +333,13 @@ k_density_alpha_div(const float4* __restrict__ posrec /* pos4 or pvx4 */, cudaTe
 //   PREDICT: out = rho*_i, kappa = max((rho* - rho0) alpha, 0), boundary term uses the boundary velocity (:136-141);
 //   else   : out = div_i (0 below 20 contacts, :62,301-314), kappa = div * alpha, boundary velocity ignored (:336-338).
 // ------------------------------------------------------------------------------------------------
-template <bool MULTI, bool PREDICT, bool TEX>
+// The v*_j gather goes through the texture pipe: 12 % faster than through LSU (profiles/r1_v1_*).
+template <bool MULTI, bool PREDICT>
 __global__ void __launch_bounds__(PASS_T, SPH_PASS_MINB)
 k_vel_divergence(const float4* __restrict__ pos, const float4* __restrict__ vs, cudaTextureObject_t tvs, const float4* __restrict__ vel,
                  const float4* __restrict__ bpos, const float4* __restrict__ bvel, Lists L, const float* __restrict__ dens,
                  const float* __restrict__ alpha, float* __restrict__ out, float* __restrict__ kappa, float* __restrict__ partial, float dt,
-                 int* __restrict__ err, const int* __restrict__ gate, uint32_t* __restrict__ ticket, float* __restrict__ errsum, Range rg) {
-    if (gate && !*gate) return;  // device-side loop control: this evaluation is past the break
+                 int* __restrict__ err, uint32_t* __restrict__ ticket, float* __restrict__ errsum, Range rg) {
     __shared__ float sm[32];
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     bool valid = i < rg.count;
@@ -403,8 +353,8 @@ k_vel_divergence(const float4* __restrict__ pos, const float4* __restrict__ vs, 
         float rho0 = C.fluids[fi].density0;
         float d = 0.f;
         if (PREDICT || L.cnt_f[i] + L.cnt_b[i] >= 20u) {
-            for_fluid_grads_pos<false>(
-                i, pi, L, pos, [&](uint32_t j) { return fetch4<TEX>(vs, tvs, j); },
+            for_fluid_grads_pos(
+                i, pi, L, pos, [&](uint32_t j) { return tex1Dfetch<float4>(tvs, (int)j); },
                 [&](uint32_t, const Pair& p, const float4& pj, const float4& vj) {
                     float dv = (vi.x - vj.x) * p.dx + (vi.y - vj.y) * p.dy + (vi.z - vj.z) * p.dz;
                     d = fmaf(dv * p.g, pj.w, d);
@@ -445,9 +395,7 @@ k_vel_divergence(const float4* __restrict__ pos, const float4* __restrict__ vs, 
 template <bool MULTI, bool BFORCE, bool PRESSURE, bool TEX>
 __global__ void __launch_bounds__(PASS_T, SPH_PASS_MINB)
 k_vel_update(const float4* __restrict__ pos, const float4* __restrict__ vel, const float4* __restrict__ bpos, Lists L, const float* __restrict__ kappa,
-             cudaTextureObject_t tkappa, float4* __restrict__ vc, float4* __restrict__ vs, float* __restrict__ bforce, float inv_dt,
-             const int* __restrict__ gate, Range rg) {
-    if (gate && !*gate) return;
+             cudaTextureObject_t tkappa, float4* __restrict__ vc, float4* __restrict__ vs, float* __restrict__ bforce, float inv_dt, Range rg) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= rg.count) return;
     i += rg.begin;
@@ -457,7 +405,7 @@ k_vel_update(const float4* __restrict__ pos, const float4* __restrict__ vel, con
     float ki = kappa[i];
     const float scale = PRESSURE ? inv_dt : 1.0f;
     float ax = 0.f, ay = 0.f, az = 0.f;
-    for_fluid_grads_pos<false>(
+    for_fluid_grads_pos(
         i, pi, L, pos, [&](uint32_t j) { return fetch1<TEX>(kappa, tkappa, j); },
         [&](uint32_t, const Pair& p, const float4& pj, float kj) {
             float c = (ki + kj) * pj.w * scale * p.g;
@@ -489,13 +437,12 @@ k_vel_update(const float4* __restrict__ pos, const float4* __restrict__ vel, con
 // and the two records of an evaluation travel through DIFFERENT data pipes (LSU / TEX).  The records are written
 // by the kernels that produce v* / kappa.  Same arithmetic as k_vel_divergence / k_vel_update.
 // ------------------------------------------------------------------------------------------------
-template <bool PREDICT, bool POS_TEX>
+template <bool PREDICT>
 __global__ void __launch_bounds__(PASS_T, SPH_PASS_MINB)
 k_vel_divergence_u(const float4* __restrict__ pvx, cudaTextureObject_t tpvx, const float2* __restrict__ vyz, cudaTextureObject_t tvyz,
                    const float4* __restrict__ bpos, const float4* __restrict__ bvel, Lists L, const float* __restrict__ dens,
                    const float* __restrict__ alpha, float* __restrict__ out, float4* __restrict__ pk4, float* __restrict__ partial, float dt,
-                   int* __restrict__ err, const int* __restrict__ gate, uint32_t* __restrict__ ticket, float* __restrict__ errsum, Range rg) {
-    if (gate && !*gate) return;
+                   int* __restrict__ err, uint32_t* __restrict__ ticket, float* __restrict__ errsum, Range rg) {
     __shared__ float sm[32];
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     bool valid = i < rg.count;
@@ -509,10 +456,10 @@ k_vel_divergence_u(const float4* __restrict__ pvx, cudaTextureObject_t tpvx, con
         const float rho0 = C.fluids[0].density0, mass = C.fluids[0].mass;
         float d = 0.f;
         if (PREDICT || L.cnt_f[i] + L.cnt_b[i] >= 20u) {
-            // POS_TEX: even contacts fetch (pvx via TEX, vyz via LSU), odd ones the other way round, so both pipes carry the same load
-            for_fluid_grads<false>(
-                i, pi, L, [&](uint32_t j, int u) { return (POS_TEX && !(u & 1)) ? tex1Dfetch<float4>(tpvx, (int)j) : __ldg(&pvx[j]); },
-                [&](uint32_t j, int u) { return (POS_TEX && !(u & 1)) ? __ldg(&vyz[j]) : tex1Dfetch<float2>(tvyz, (int)j); },
+            // even contacts fetch (pvx via TEX, vyz via LSU), odd ones the other way round, so both pipes carry the same load
+            for_fluid_grads(
+                i, pi, L, [&](uint32_t j, int u) { return !(u & 1) ? tex1Dfetch<float4>(tpvx, (int)j) : __ldg(&pvx[j]); },
+                [&](uint32_t j, int u) { return !(u & 1) ? __ldg(&vyz[j]) : tex1Dfetch<float2>(tvyz, (int)j); },
                 [&](uint32_t, const Pair& p, const float4& pj, const float2& wj) {
                     float dv = (vix - pj.w) * p.dx + (viy - wj.x) * p.dy + (viz - wj.y) * p.dz;
                     d = fmaf(dv * p.g, mass, d);
@@ -546,220 +493,6 @@ k_vel_divergence_u(const float4* __restrict__ pvx, cudaTextureObject_t tpvx, con
     reduce_error<false>(e, 0u, valid, partial, sm, ticket, errsum);
 }
 
-// ------------------------------------------------------------------------------------------------
-// 256-bit gather records (sm_100 LDG.E.256): rec8[i] = (x, y, z, v*x, v*y, v*z, rho, unused), 32-byte aligned, so an
-// evaluation pays ONE gather instruction per contact instead of two (position record + velocity record).  The gather
-// passes are bound by L1TEX wavefronts (one per distinct 128-byte line a warp-wide gather touches, ~8 per instruction,
-// profiles/r1_*), not by bytes: halving the gather instructions per contact is what moves them.
-// ------------------------------------------------------------------------------------------------
-// EXTRA selects what rides with a stand-alone divergence evaluation (PREDICT = false only):
-//   1: the fluid term of XSPHViscosity::solve (xsph_viscosity.rs:52-69; valid when this is the loop's LAST evaluation, see
-//      k_vel_divergence_xsph_u) -> xs;   2: Akinci2013 compute_normals (akinci2013_surface_tension.rs:43-68: positions and
-//      densities only, so ANY evaluation of the step may produce them) -> nrec = (x, y, z, n_x, n_y, n_z, rho, -), the
-//      one-gather record of the force pass.  rho_j comes with the record: no extra gather.
-template <bool PREDICT, int EXTRA>
-__global__ void __launch_bounds__(PASS_T, EXTRA ? SPH_FORCE_MINB : SPH_PASS_MINB)  // the extra sums spill at 56 registers
-k_vel_divergence_r8(const Rec8* __restrict__ rec, const float4* __restrict__ bpos, const float4* __restrict__ bvel, Lists L, const float* __restrict__ dens,
-                    const float* __restrict__ alpha, float* __restrict__ out, float4* __restrict__ pk4, float* __restrict__ partial, float dt,
-                    int* __restrict__ err, uint32_t* __restrict__ ticket, float* __restrict__ errsum, float4* __restrict__ xs, float cf,
-                    Rec8* __restrict__ nrec, Range rg) {
-    __shared__ float sm[32];
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    bool valid = i < rg.count;
-    i += rg.begin;
-    float e = 0.f;
-    if (valid) {
-        float4 a, b;
-        ld_rec8(rec + i, a, b);
-        const float4 pi = make_float4(a.x, a.y, a.z, 0.f);
-        const float vix = a.w, viy = b.x, viz = b.y;
-        const float rho0 = C.fluids[0].density0, mass = C.fluids[0].mass;
-        float d = 0.f, ex = 0.f, ey = 0.f, ez = 0.f;
-        const bool gated = !PREDICT && L.cnt_f[i] + L.cnt_b[i] < 20u;  // dfsph_solver.rs:301-314
-        if (!gated || EXTRA) {
-            const uint32_t n = min(L.cnt_f[i], C.cap_f);
-            const uint32_t nq = (n + 3u) >> 2;
-            const uint4* col = L.nbr_f + i;
-            uint4 J = nq ? ld_list(col) : make_uint4(i, i, i, i);
-            for (uint32_t q = 0; q < nq; ++q) {
-                uint4 Jn = J;
-                if (q + 1 < nq) Jn = ld_list(col + (size_t)(q + 1) * C.stride);
-                const uint32_t j[4] = {J.x, J.y, J.z, J.w};
-                float4 pj[4], wj[4];
-#pragma unroll
-                for (int u = 0; u < 4; ++u) ld_rec8(rec + j[u], pj[u], wj[u]);
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {  // padded tail slots are self contacts: zero gradient, zero velocity difference
-                    Pair p = make_pair<EXTRA == 1, true>(pi, pj[u]);
-                    float dv = (vix - pj[u].w) * p.dx + (viy - wj[u].x) * p.dy + (viz - wj[u].y) * p.dz;
-                    d = fmaf(dv * p.g, mass, d);
-                    if (EXTRA == 1) {
-                        float c = cf * p.w * mass / wj[u].z;  // coeff * W * (vol_j * rho0) / rho_j
-                        ex = fmaf(c, pj[u].w - vix, ex); ey = fmaf(c, wj[u].x - viy, ey); ez = fmaf(c, wj[u].y - viz, ez);
-                    } else if (EXTRA == 2) {
-                        float c = p.g * (mass / wj[u].z);
-                        ex = fmaf(c, p.dx, ex); ey = fmaf(c, p.dy, ey); ez = fmaf(c, p.dz, ez);
-                    }
-                }
-                J = Jn;
-            }
-            if (gated) d = 0.f;
-            else
-                for_boundary_contacts<false, true>(i, pi, L, bpos, [&](uint32_t j, const Pair& p, const float4& pj) {
-                    float dv;
-                    if (PREDICT) {
-                        float4 vj = __ldg(&bvel[j]);
-                        dv = (vix - vj.x) * p.dx + (viy - vj.y) * p.dy + (viz - vj.z) * p.dz;
-                    } else {
-                        dv = vix * p.dx + viy * p.dy + viz * p.dz;
-                    }
-                    d = fmaf(dv * p.g, pj.w * rho0, d);
-                });
-        }
-        float kap;
-        if (PREDICT) {
-            float pd = fmaf(d, dt, dens[i]);
-            if (pd == 0.f) atomicOr(err, 1);
-            out[i] = pd;
-            kap = fmaxf((pd - rho0) * alpha[i], 0.f);
-            e = pd < rho0 ? 0.f : pd / rho0 - 1.0f;
-        } else {
-            d = fmaxf(d, 0.f);
-            out[i] = d;
-            kap = d * alpha[i];
-            e = d / rho0;
-        }
-        pk4[i] = make_float4(a.x, a.y, a.z, kap);
-        if (EXTRA == 1) xs[i] = make_float4(ex, ey, ez, 0.f);
-        if (EXTRA == 2) st_rec8(nrec + i, a.x, a.y, a.z, ex * C.h, ey * C.h, ez * C.h, b.z);
-    }
-    reduce_error<false>(e, 0u, valid, partial, sm, ticket, errsum);
-}
-
-// K3 + first K4a on the 256-bit records (k_density_alpha_div with ONE gather per contact).
-__global__ void __launch_bounds__(PASS_T, SPH_FORCE_MINB)
-k_density_alpha_div_r8(const Rec8* __restrict__ rec, const float4* __restrict__ bpos, Lists L, float* __restrict__ dens, float* __restrict__ alpha,
-                       float* __restrict__ divv, float4* __restrict__ pk4, float* __restrict__ partial, int* __restrict__ err, uint32_t* __restrict__ ticket,
-                       float* __restrict__ errsum, Range rg) {
-    __shared__ float sm[32];
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    bool valid = i < rg.count;
-    i += rg.begin;
-    float e = 0.f;
-    if (valid) {
-        float4 a, b;
-        ld_rec8(rec + i, a, b);
-        const float4 pi = make_float4(a.x, a.y, a.z, 0.f);
-        const float vix = a.w, viy = b.x, viz = b.y;
-        const float rho0 = C.fluids[0].density0, umass = C.fluids[0].mass;
-        float rho = 0.f, sq = 0.f, gx = 0.f, gy = 0.f, gz = 0.f, d = 0.f;
-        const uint32_t n = min(L.cnt_f[i], C.cap_f);
-        const uint32_t nq = (n + 3u) >> 2;
-        const uint4* col = L.nbr_f + i;
-        uint4 J = nq ? ld_list(col) : make_uint4(i, i, i, i);
-        for (uint32_t q = 0; q < nq; ++q) {
-            uint4 Jn = J;
-            if (q + 1 < nq) Jn = ld_list(col + (size_t)(q + 1) * C.stride);
-            const uint32_t j[4] = {J.x, J.y, J.z, J.w};
-            float4 pj[4], wj[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) ld_rec8(rec + j[u], pj[u], wj[u]);
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                if (q * 4u + u < n) {  // tail slots point at i itself and would add W(0) again
-                    Pair p = make_pair<true, true>(pi, pj[u]);
-                    rho = fmaf(umass, p.w, rho);
-                    float s = p.g * umass;  // m_j * gradient
-                    float ax = s * p.dx, ay = s * p.dy, az = s * p.dz;
-                    sq += ax * ax + ay * ay + az * az;
-                    gx += ax; gy += ay; gz += az;
-                    float dv = (vix - pj[u].w) * p.dx + (viy - wj[u].x) * p.dy + (viz - wj[u].y) * p.dz;
-                    d = fmaf(dv * p.g, umass, d);
-                }
-            }
-            J = Jn;
-        }
-        for_boundary_contacts<true, true>(i, pi, L, bpos, [&](uint32_t, const Pair& p, const float4& pj) {
-            float mb = pj.w * rho0;  // boundary pseudo mass: vol_b * rho0_i
-            rho = fmaf(mb, p.w, rho);
-            float s = p.g * mb;
-            float ax = s * p.dx, ay = s * p.dy, az = s * p.dz;
-            sq += ax * ax + ay * ay + az * az;
-            gx += ax; gy += ay; gz += az;
-            float dv = vix * p.dx + viy * p.dy + viz * p.dz;  // boundary velocity ignored (dfsph_solver.rs:336-338)
-            d = fmaf(dv * p.g, mb, d);
-        });
-        if (rho == 0.f) atomicOr(err, 1);  // assert!(!density.is_zero()) dfsph_solver.rs:662
-        float den = sq + (gx * gx + gy * gy + gz * gz);
-        float al = den <= 1.0e-5f ? 0.f : 1.0f / den;  // dfsph_solver.rs:209-213
-        dens[i] = rho;
-        alpha[i] = al;
-        if (L.cnt_f[i] + L.cnt_b[i] < 20u) d = 0.f;  // min_neighbors_for_divergence_solve :62,301-314
-        d = fmaxf(d, 0.f);
-        divv[i] = d;
-        pk4[i] = make_float4(a.x, a.y, a.z, d * al);
-        e = d / rho0;
-    }
-    reduce_error<false>(e, 0u, valid, partial, sm, ticket, errsum);
-}
-
-// a14 pass 2 on the one-gather record nrec = (x, y, z, n_x, n_y, n_z, rho, -) written by k_vel_divergence_r8<false, 2>:
-// Akinci2013SurfaceTension::solve akinci2013_surface_tension.rs:113-192, single fluid.
-template <bool BFORCE>
-__global__ void __launch_bounds__(PASS_T, SPH_FORCE_MINB)
-k_akinci_force_r8(const Rec8* __restrict__ nrec, const float4* __restrict__ bpos, Lists L, float4* __restrict__ acc, float* __restrict__ bforce, float gamma,
-                  float adh, float coh_norm, float h6_64, float adh_norm) {
-    SPH_OWNED_INDEX(i)
-    float4 a, b;
-    ld_rec8(nrec + i, a, b);
-    const float4 pi = make_float4(a.x, a.y, a.z, C.fluids[0].mass);
-    const float rho0 = C.fluids[0].density0, mass = C.fluids[0].mass;
-    const float nix = a.w, niy = b.x, niz = b.y, rho_i = b.z;
-    float ax = 0.f, ay = 0.f, az = 0.f;
-    if (gamma != 0.f) {
-        const uint32_t n = min(L.cnt_f[i], C.cap_f);
-        const uint32_t nq = (n + 3u) >> 2;
-        const uint4* col = L.nbr_f + i;
-        uint4 J = nq ? ld_list(col) : make_uint4(i, i, i, i);
-        for (uint32_t q = 0; q < nq; ++q) {
-            uint4 Jn = J;
-            if (q + 1 < nq) Jn = ld_list(col + (size_t)(q + 1) * C.stride);
-            const uint32_t j[4] = {J.x, J.y, J.z, J.w};
-            float4 pj[4], wj[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) ld_rec8(nrec + j[u], pj[u], wj[u]);
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                if (q * 4u + u < n) {
-                    Pair p = make_pair<false, false>(pi, pj[u]);
-                    // cohesion_vec = dir * C(dist) if |dpos|^2 > eps^2 (Unit::try_new_and_get)
-                    float coh = p.d2 > F32_EPS * F32_EPS ? cohesion_kernel(p.r, coh_norm, h6_64) / p.r : 0.f;
-                    float cm = coh * (-gamma * mass);
-                    float kij = 2.0f * rho0 / (rho_i + wj[u].z);
-                    ax += (-gamma * (nix - pj[u].w) + cm * p.dx) * kij;
-                    ay += (-gamma * (niy - wj[u].x) + cm * p.dy) * kij;
-                    az += (-gamma * (niz - wj[u].y) + cm * p.dz) * kij;
-                }
-            }
-            J = Jn;
-        }
-    }
-    if (adh != 0.f)
-        for_boundary_contacts<false, false>(i, pi, L, bpos, [&](uint32_t j, const Pair& p, const float4& pj) {
-            float ad = p.d2 > F32_EPS * F32_EPS ? adhesion_kernel(p.r, adh_norm) / p.r : 0.f;
-            float c = ad * adh * (pj.w * rho0);
-            ax -= c * p.dx; ay -= c * p.dy; az -= c * p.dz;
-            if (BFORCE) {  // apply_force(c.j, adhesion_acc * m_i) :188
-                atomicAdd(&bforce[3 * (size_t)j + 0], c * p.dx * mass);
-                atomicAdd(&bforce[3 * (size_t)j + 1], c * p.dy * mass);
-                atomicAdd(&bforce[3 * (size_t)j + 2], c * p.dz * mass);
-            }
-        });
-    float4 o = acc[i];
-    o.x += ax; o.y += ay; o.z += az;
-    acc[i] = o;
-}
-
 // compute_divergences (a7) + the fluid term of XSPHViscosity::solve (a12, xsph_viscosity.rs:52-69) in ONE sweep.
 // XSPH is evaluated on `fluid.velocities` right after update_velocities folded vc into them (dfsph_solver.rs:688-697),
 // i.e. on exactly the v* the divergence loop's LAST evaluation gathers; so every stand-alone evaluation also accumulates
@@ -774,7 +507,7 @@ struct VyzRho {
 // instead: n_i = h sum_j (m_j / rho_j) grad W_ij needs positions and densities only, so ANY stand-alone evaluation of the
 // step may produce it; the output record nr4 = (n_x, n_y, n_z, rho_i) is what k_akinci_force_u gathers (one float4 instead
 // of a normal and a density), and the separate normals pass is skipped.
-template <bool POS_TEX, int EXTRA>
+template <int EXTRA>
 __global__ void __launch_bounds__(PASS_T, SPH_FORCE_MINB)  // 64 registers: the extra sums spill at 56
 k_vel_divergence_xsph_u(const float4* __restrict__ pvx, cudaTextureObject_t tpvx, const float2* __restrict__ vyz, cudaTextureObject_t tvyz,
                         const float4* __restrict__ bpos, Lists L, const float* __restrict__ dens, const float* __restrict__ alpha,
@@ -793,9 +526,9 @@ k_vel_divergence_xsph_u(const float4* __restrict__ pvx, cudaTextureObject_t tpvx
         const float rho0 = C.fluids[0].density0, mass = C.fluids[0].mass;
         const bool gated = L.cnt_f[i] + L.cnt_b[i] < 20u;  // dfsph_solver.rs:301-314
         float d = 0.f, fx = 0.f, fy = 0.f, fz = 0.f;
-        for_fluid_grads<false, EXTRA == 1>(
-            i, pi, L, [&](uint32_t j, int u) { return (POS_TEX && !(u & 1)) ? tex1Dfetch<float4>(tpvx, (int)j) : __ldg(&pvx[j]); },
-            [&](uint32_t j, int u) { return VyzRho{(POS_TEX && !(u & 1)) ? __ldg(&vyz[j]) : tex1Dfetch<float2>(tvyz, (int)j), __ldg(&dens[j])}; },
+        for_fluid_grads<EXTRA == 1>(
+            i, pi, L, [&](uint32_t j, int u) { return !(u & 1) ? tex1Dfetch<float4>(tpvx, (int)j) : __ldg(&pvx[j]); },
+            [&](uint32_t j, int u) { return VyzRho{!(u & 1) ? __ldg(&vyz[j]) : tex1Dfetch<float2>(tvyz, (int)j), __ldg(&dens[j])}; },
             [&](uint32_t, const Pair& p, const float4& pj, const VyzRho& wj) {
                 float dv = (vix - pj.w) * p.dx + (viy - wj.v.x) * p.dy + (viz - wj.v.y) * p.dz;
                 d = fmaf(dv * p.g, mass, d);
@@ -867,14 +600,13 @@ k_akinci_force_u(const float4* __restrict__ pvx, cudaTextureObject_t tpvx, const
     acc[i] = o;
 }
 
-// POS_TEX: the (x, y, z, kappa) gather goes through the texture pipe (true) or the LSU pipe (false).  ALT (runtime, uniform):
-// contacts 0 and 2 of every group of four through TEX, 1 and 3 through LSU, so both L1TEX front ends carry half the wavefronts.
-template <bool BFORCE, bool PRESSURE, bool POS_TEX>
+// The (x, y, z, kappa) gathers of every group of four contacts are split between the two L1TEX front ends: contacts 0 and 2
+// through the texture pipe, 1 and 3 through the LSU pipe, so both carry half the wavefronts.
+template <bool BFORCE, bool PRESSURE>
 __global__ void __launch_bounds__(PASS_T, SPH_PASS_MINB)
 k_vel_update_u(const float4* __restrict__ pk4, cudaTextureObject_t tpk, const float4* __restrict__ vel, const float4* __restrict__ bpos, Lists L,
-               float4* __restrict__ vc, float4* __restrict__ vs, float4* __restrict__ pvx, float2* __restrict__ vyz, Rec8* __restrict__ rec,
-               const float* __restrict__ dens, float* __restrict__ bforce, float inv_dt, const int* __restrict__ gate, Range rg) {
-    if (gate && !*gate) return;
+               float4* __restrict__ vc, float4* __restrict__ vs, float4* __restrict__ pvx, float2* __restrict__ vyz, float* __restrict__ bforce,
+               float inv_dt, Range rg) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= rg.count) return;
     i += rg.begin;
@@ -885,77 +617,12 @@ k_vel_update_u(const float4* __restrict__ pk4, cudaTextureObject_t tpk, const fl
     const float rho0 = C.fluids[0].density0, mass = C.fluids[0].mass;
     const float scale = (PRESSURE ? inv_dt : 1.0f) * mass;
     float ax = 0.f, ay = 0.f, az = 0.f;
-    for_fluid_grads<false>(
-        i, pi, L, [&](uint32_t j, int u) { return (POS_TEX && !(u & 1)) ? tex1Dfetch<float4>(tpk, (int)j) : __ldg(&pk4[j]); }, [](uint32_t) { return NoAux{}; },
+    for_fluid_grads(
+        i, pi, L, [&](uint32_t j, int u) { return !(u & 1) ? tex1Dfetch<float4>(tpk, (int)j) : __ldg(&pk4[j]); }, [](uint32_t) { return NoAux{}; },
         [&](uint32_t, const Pair& p, const float4& pj, NoAux) {
             float c = (ki + pj.w) * scale * p.g;
             ax = fmaf(c, p.dx, ax); ay = fmaf(c, p.dy, ay); az = fmaf(c, p.dz, az);
         });
-    if (!PRESSURE || ki > 0.f) {
-        const float bscale = PRESSURE ? inv_dt : 1.0f;
-        for_boundary_contacts<false, true>(i, pi, L, bpos, [&](uint32_t j, const Pair& p, const float4& pj) {
-            float c = ki * pj.w * rho0 * bscale * p.g;
-            ax = fmaf(c, p.dx, ax); ay = fmaf(c, p.dy, ay); az = fmaf(c, p.dz, az);
-            if (BFORCE) {
-                float s = c * inv_dt * mass;
-                atomicAdd(&bforce[3 * (size_t)j + 0], s * p.dx);
-                atomicAdd(&bforce[3 * (size_t)j + 1], s * p.dy);
-                atomicAdd(&bforce[3 * (size_t)j + 2], s * p.dz);
-            }
-        });
-    }
-    float4 c4 = vc[i];
-    c4.x -= ax; c4.y -= ay; c4.z -= az;
-    vc[i] = c4;
-    const float sx = v.x + c4.x, sy = v.y + c4.y, sz = v.z + c4.z;
-    vs[i] = make_float4(sx, sy, sz, 0.f);
-    if (rec) {
-        st_rec8(rec + i, a.x, a.y, a.z, sx, sy, sz, dens[i]);
-    } else {
-        pvx[i] = make_float4(a.x, a.y, a.z, sx);
-        vyz[i] = make_float2(sy, sz);
-    }
-}
-
-// k_vel_update_u with the gathers of every group of four contacts split between the two L1TEX front ends: contacts 0 and 2
-// through the texture pipe, 1 and 3 through the LSU pipe (SALVA_B200_UNI_UPD=3).  Same arithmetic and summation order.
-template <bool BFORCE, bool PRESSURE>
-__global__ void __launch_bounds__(PASS_T, SPH_PASS_MINB)
-k_vel_update_alt(const float4* __restrict__ pk4, cudaTextureObject_t tpk, const float4* __restrict__ vel, const float4* __restrict__ bpos, Lists L,
-                 float4* __restrict__ vc, float4* __restrict__ vs, float4* __restrict__ pvx, float2* __restrict__ vyz, float* __restrict__ bforce, float inv_dt,
-                 Range rg) {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= rg.count) return;
-    i += rg.begin;
-    const float4 a = pk4[i];
-    const float4 pi = make_float4(a.x, a.y, a.z, 0.f);
-    const float ki = a.w;
-    const float4 v = vel[i];
-    const float rho0 = C.fluids[0].density0, mass = C.fluids[0].mass;
-    const float scale = (PRESSURE ? inv_dt : 1.0f) * mass;
-    float ax = 0.f, ay = 0.f, az = 0.f;
-    {
-        const uint32_t n = min(L.cnt_f[i], C.cap_f);
-        const uint32_t nq = (n + 3u) >> 2;
-        const uint4* col = L.nbr_f + i;
-        uint4 J = nq ? ld_list(col) : make_uint4(i, i, i, i);
-        for (uint32_t q = 0; q < nq; ++q) {
-            uint4 Jn = J;
-            if (q + 1 < nq) Jn = ld_list(col + (size_t)(q + 1) * C.stride);
-            float4 pj[4];
-            pj[0] = tex1Dfetch<float4>(tpk, (int)J.x);
-            pj[1] = __ldg(&pk4[J.y]);
-            pj[2] = tex1Dfetch<float4>(tpk, (int)J.z);
-            pj[3] = __ldg(&pk4[J.w]);
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {  // padded tail slots are self contacts: zero gradient
-                Pair p = make_pair<false, true>(pi, pj[u]);
-                float c = (ki + pj[u].w) * scale * p.g;
-                ax = fmaf(c, p.dx, ax); ay = fmaf(c, p.dy, ay); az = fmaf(c, p.dz, az);
-            }
-            J = Jn;
-        }
-    }
     if (!PRESSURE || ki > 0.f) {
         const float bscale = PRESSURE ? inv_dt : 1.0f;
         for_boundary_contacts<false, true>(i, pi, L, bpos, [&](uint32_t j, const Pair& p, const float4& pj) {
@@ -1040,7 +707,7 @@ k_force_artificial(const float4* __restrict__ pos, const float4* __restrict__ ve
     float eta2 = C.h * C.h * 0.01f;
     float fx = 0.f, fy = 0.f, fz = 0.f, bx = 0.f, by = 0.f, bz = 0.f;
     if (cf != 0.f)
-        for_fluid_grads_pos<true>(
+        for_fluid_grads_pos(
             i, pi, L, pos, [&](uint32_t j) { return VelRho{__ldg(&vel[j]), __ldg(&dens[j])}; },
             [&](uint32_t, const Pair& p, const float4& pj, const VelRho& a) {
                 if (MULTI && fid_of(a.v) != which) return;
@@ -1085,7 +752,7 @@ k_akinci_normals(const float4* __restrict__ pos, const float4* __restrict__ vel,
     if (MULTI && fid_of(vel[i]) != which) return;
     float4 pi = pos[i];
     float nx = 0.f, ny = 0.f, nz = 0.f;
-    for_fluid_grads_pos<false>(
+    for_fluid_grads_pos(
         i, pi, L, pos, [&](uint32_t j) { return FidRho{MULTI ? fid_of(__ldg(&vel[j])) : 0u, __ldg(&dens[j])}; },
         [&](uint32_t, const Pair& p, const float4& pj, const FidRho& a) {
             if (MULTI && a.fid != which) return;
@@ -1177,7 +844,7 @@ k_he2014_gradc(const float4* __restrict__ pos, const float4* __restrict__ vel, L
     if (MULTI && fid_of(vel[i]) != which) return;
     float4 pi = pos[i];
     float gx = 0.f, gy = 0.f, gz = 0.f;
-    for_fluid_grads_pos<false>(
+    for_fluid_grads_pos(
         i, pi, L, pos, [&](uint32_t j) { return FidRhoVal{MULTI ? fid_of(__ldg(&vel[j])) : 0u, __ldg(&dens[j]), __ldg(&colors[j])}; },
         [&](uint32_t, const Pair& p, const float4& pj, const FidRhoVal& a) {
             if (MULTI && a.fid != which) return;
@@ -1202,7 +869,7 @@ k_he2014_force(const float4* __restrict__ pos, const float4* __restrict__ vel, c
     float ax = 0.f, ay = 0.f, az = 0.f;
     if (cf != 0.f) {
         const float k = cf / (2.0f * mi);
-        for_fluid_grads_pos<false>(
+        for_fluid_grads_pos(
             i, pi, L, pos, [&](uint32_t j) { return FidRhoVal{MULTI ? fid_of(__ldg(&vel[j])) : 0u, __ldg(&dens[j]), __ldg(&gradc[j])}; },
             [&](uint32_t, const Pair& p, const float4& pj, const FidRhoVal& a) {
                 if (MULTI && a.fid != which) return;

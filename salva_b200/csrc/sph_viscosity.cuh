@@ -119,7 +119,7 @@ k_visc_betas(const float4* __restrict__ pos, const float4* __restrict__ vel, Lis
     const float rho_i = dens[i];
     Sym15 sq = {};
     float A = 0.f, B = 0.f, Cz = 0.f, SX = 0.f, SY = 0.f, SZ = 0.f;
-    for_fluid_grads_pos<false>(
+    for_fluid_grads_pos(
         i, pi, L, pos, [&](uint32_t j) { return MULTI ? fid_of(__ldg(&vel[j])) : 0u; },
         [&](uint32_t, const Pair& p, const float4& pj, uint32_t fj) {
             if (MULTI && fj != which) return;
@@ -177,7 +177,7 @@ k_visc_rates(const float4* __restrict__ pos, const float4* __restrict__ vel, Lis
         const float rho_i = dens[i];
         const float4 vi = vv[i];
         float r0 = 0.f, r1 = 0.f, r2 = 0.f, r3 = 0.f, r4 = 0.f, r5 = 0.f;
-        for_fluid_grads_pos<false>(
+        for_fluid_grads_pos(
             i, pi, L, pos, [&](uint32_t j) { return __ldg(&vv[j]); },
             [&](uint32_t, const Pair& p, const float4& pj, const float4& vj) {
                 if (MULTI && fid_of(vj) != which) return;
@@ -232,7 +232,7 @@ k_visc_accel(const float4* __restrict__ pos, const float4* __restrict__ vel, Lis
     const float2 ub = u2[i];
     const float k = pi.w * inv_dt;  // volumes[c.i] * density0 * inv_dt
     float ax = 0.f, ay = 0.f, az = 0.f;
-    for_fluid_grads_pos<false>(
+    for_fluid_grads_pos(
         i, pi, L, pos, [&](uint32_t j) { return U6{__ldg(&u4[j]), __ldg(&u2[j]), MULTI ? fid_of(__ldg(&vel[j])) : 0u}; },
         [&](uint32_t, const Pair& p, const float4& pj, const U6& uj) {
             if (MULTI && uj.fid != which) return;

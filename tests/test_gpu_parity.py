@@ -168,10 +168,9 @@ def test_dfsph_viscosity_coefficient_range_is_checked():
         gpu.push_force(f, *scenes.dfsph_viscosity(1.5))
 
 
-def test_xsph_fusion_falls_back_when_the_loop_ends_with_an_update(monkeypatch):
+def test_xsph_fusion_falls_back_when_the_loop_ends_with_an_update():
     """divergence_solve that runs out of iterations ends with an UPDATE (dfsph_solver.rs:474-502): the XSPH sums of its
     last evaluation are stale, so the separate XSPH pass must run."""
-    monkeypatch.setenv("SALVA_B200_FUSE_XSPH", "1")
     sc = _small_scene(seed=41, forces=(scenes.xsph_viscosity(0.5, 0.0),))
     solver = DFSPHSolver()
     solver.max_divergence_iter, solver.max_divergence_error = 2, 1e-9      # never converges: exactly 2 updates
@@ -193,11 +192,10 @@ def test_xsph_fusion_falls_back_when_the_loop_ends_with_an_update(monkeypatch):
 
 
 @pytest.mark.parametrize("mode", ["forced", "free", "boundary-term-fallback"])
-def test_xsph_fused_with_divergence_evaluation(mode, monkeypatch):
-    """SALVA_B200_FUSE_XSPH=1: the XSPH sums ride with the divergence loop's stand-alone evaluations
+def test_xsph_fused_with_divergence_evaluation(mode):
+    """The XSPH sums ride with the divergence loop's stand-alone evaluations
     (k_vel_divergence_xsph_u) and k_fold_velocities applies the last ones; with a boundary coefficient the engine must
     fall back to the separate pass.  Same tolerances as the plain trajectory test."""
-    monkeypatch.setenv("SALVA_B200_FUSE_XSPH", "1")
     forces = (scenes.xsph_viscosity(0.5, 0.3 if mode == "boundary-term-fallback" else 0.0),)
     sc = _small_scene(seed=37, forces=forces)
     gpu, cpu, fg, fc, _, _ = _pair(sc)

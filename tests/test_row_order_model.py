@@ -1,46 +1,22 @@
 """CPU model of the whole "row order" neighbour search (salva_b200/csrc: phase_grid dims, k_cell_hist_xy, k_neighbors_xy with
-arun() / zrun()), in numpy f32, against a brute-force statement of the reference's rule (contacts.rs:154-400: pairs of the
+arun()), in numpy f32, against a brute-force statement of the reference's rule (contacts.rs:154-400: pairs of the
 3 x 3 x 3 cells floor(x / h) +- 1 that pass `(dx*dx + dy*dy) + dz*dz <= h*h`).
 
 The CUDA kernels of this mode could not be run when they were written (no GPU minutes left), so everything that is pure index
 arithmetic — bin functions, grid origin / dims with one padding cell, row ranges, run bounds into the exclusive-scanned cell table,
 ascending list order — is restated here line by line and checked for random clouds and jittered lattices, with sub-division factors
-1 (plain cells), 2 (the mode bench.py probes) and 3.
+1 (plain cells), 2 (the mode bench.py probes), 3 and 4 (the largest the engine accepts).
 """
 import numpy as np
 import pytest
 
-from test_zbin_model import F, _round_dir, zbin
+from test_zbin_model import F, abin, arun
 
 # ---- device helpers (sph_kernels.cuh) ------------------------------------------------------------------------------------
 
 
 def cell_coord(v, h):
     return int(np.floor(F(v) / F(h)))
-
-
-def abin(v, h, sub):
-    q = F(v) / F(h)
-    fl = np.floor(q)
-    return int(fl) * sub + min(sub - 1, int(F(q - fl) * F(sub)))
-
-
-def h_reach(h):
-    return np.nextafter(F(F(h) * F(1.00001)), F(np.inf))
-
-
-def arun(v, c, h, sub):
-    lo = max(abin(_round_dir(float(F(v)) - float(h_reach(h)), up=False), h, sub), (c - 1) * sub)
-    hi = min(abin(_round_dir(float(F(v)) + float(h_reach(h)), up=True), h, sub), (c + 2) * sub - 1)
-    return lo, hi
-
-
-def zrun(z, cz, h, zsub):
-    if zsub == 1:
-        return cz - 1, cz + 1
-    lo = max(zbin(_round_dir(float(F(z)) - float(h_reach(h)), up=False), h, zsub), (cz - 1) * zsub)
-    hi = min(zbin(_round_dir(float(F(z)) + float(h_reach(h)), up=True), h, zsub), (cz + 2) * zsub - 1)
-    return lo, hi
 
 
 def accepted(a, b, h):
@@ -52,20 +28,20 @@ def accepted(a, b, h):
 # ---- the search as the engine runs it ------------------------------------------------------------------------------------
 
 
-def row_order_search(pts, h, xysub, zsub):
+def row_order_search(pts, h, xysub):
     n = len(pts)
     cells = np.array([[cell_coord(p[a], h) for a in range(3)] for p in pts])
     lo_c, hi_c = cells.min(axis=0), cells.max(axis=0)                 # k_bounds
     dims = hi_c - lo_c + 3                                            # phase_grid: one padding cell each side
-    ox, oy, oz = (lo_c[0] - 1) * xysub, (lo_c[1] - 1) * xysub, (lo_c[2] - 1) * zsub
-    nx, ny, nz = dims[0] * xysub, dims[1] * xysub, dims[2] * zsub
+    ox, oy, oz = (lo_c[0] - 1) * xysub, (lo_c[1] - 1) * xysub, lo_c[2] - 1
+    nx, ny, nz = dims[0] * xysub, dims[1] * xysub, dims[2]
     ncell = nx * ny * nz
 
     def cell_id(bx, by, bz):
         return ((bx - ox) * ny + (by - oy)) * nz + (bz - oz)
 
     ids = np.array([cell_id(abin(p[0], h, xysub) if xysub > 1 else cell_coord(p[0], h),
-                            abin(p[1], h, xysub) if xysub > 1 else cell_coord(p[1], h), zbin(p[2], h, zsub)) for p in pts])  # k_cell_hist(_xy)
+                            abin(p[1], h, xysub) if xysub > 1 else cell_coord(p[1], h), cell_coord(p[2], h)) for p in pts])  # k_cell_hist(_xy)
     assert ids.min() >= 0 and ids.max() < ncell
     order = np.lexsort((np.arange(n), ids))                           # counting sort + canonical in-cell order (ascending id)
     spts = pts[order]
@@ -81,7 +57,7 @@ def row_order_search(pts, h, xysub, zsub):
             ylo, yhi = arun(pi[1], cy, h, xysub)
         else:
             xlo, xhi, ylo, yhi = cx - 1, cx + 1, cy - 1, cy + 1
-        zlo, zhi = zrun(pi[2], cz, h, zsub)
+        zlo, zhi = cz - 1, cz + 1
         out = []
         for bx in range(xlo, xhi + 1):
             for by in range(ylo, yhi + 1):
@@ -122,12 +98,12 @@ def _lattice(seed, h):
     return (p + rng.uniform(-0.05 * r, 0.05 * r, p.shape) - 1.3 * h).astype(F)   # marginal neighbours at d ~ h, negative coordinates
 
 
-@pytest.mark.parametrize("xysub,zsub", [(1, 1), (2, 1), (2, 2), (3, 1)])
+@pytest.mark.parametrize("xysub", [1, 2, 3, 4])
 @pytest.mark.parametrize("kind", ["cloud", "lattice"])
-def test_row_order_search_finds_exactly_the_reference_contacts(xysub, zsub, kind):
+def test_row_order_search_finds_exactly_the_reference_contacts(xysub, kind):
     h = 0.1
     pts = _cloud(5 + xysub, 260, h, 1.6) if kind == "cloud" else _lattice(3, h)
-    got = row_order_search(pts, h, xysub, zsub)
+    got = row_order_search(pts, h, xysub)
     want = brute_force(pts, h)
     assert got == want
     assert sum(len(s) for s in want) > 4 * len(pts)                   # the scenes do have contacts
